@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- instance-field render throughput (BASELINE.json metric: Mrays/s; train-step ms @ 4096 rays) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload render|c4|train] [--rays R]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload render|c4|train] [--rays R] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload of the headline line (BASELINE.json configs[1], SURVEY.md section 8d "c2"): 640x480 frames (307 200 rays each) of the
@@ -32,6 +32,10 @@ Keys of the JSON line:
   ref_cuda_path the reference's own CUDA kernels (oracle/_ref) on c2 and c3, timed in a subprocess (BASELINE.md B2)
 
 --impl reference runs ONLY the CPU path (the reference arm): no CUDA code of this repo is touched.
+
+--dump-outputs DIR (render workload) writes what NeRFNetwork.render returned in the last device-resident timed step -- on rank 0,
+its own rows at N > 1 -- as DIR/<key>.npy (image, depth, instance_mask_logits; float32, 44 MB at K=32).  The inputs depend
+only on the arguments, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -325,6 +329,7 @@ def run_gpu_arm(args):
                 copy_done[b].record()
         else:
             gather.submit(tile)
+        return r
 
     def drain():
         gather.drain()
@@ -357,7 +362,7 @@ def run_gpu_arm(args):
         flush_buf.fill_(i & 0xFF)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        step(args.warmup + i)
+        last = step(args.warmup + i)
         if i == args.steps - 1:
             drain()
         e1.record()
@@ -365,6 +370,9 @@ def run_gpu_arm(args):
     barrier()
     torch.cuda.nvtx.range_pop()
     wall_s = time.perf_counter() - t_wall0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     total_ms = sum(a.elapsed_time(b) for a, b in ev)
     kern_ms = [a.elapsed_time(b) for a, b in kern_events]
     n_samples = [int(s[2:4].view(torch.int64).item()) for s in samples_seen]
@@ -517,6 +525,18 @@ def run_gpu_arm(args):
         emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, results):
+    """results (a dict of [1, N, ...] device tensors, None for absent keys) -> out_dir/<key>.npy, float32."""
+    import numpy as np
+    arrays = {k: v[0].float().cpu().numpy() for k, v in results.items() if v is not None}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} B, more than 64 MB")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def run_ref_cuda_subprocess():
@@ -815,9 +835,15 @@ def main():
                     help="render = the headline metric on c2 (default); c4 = 200 poses x 1920x1080; train = train-step ms")
     ap.add_argument("--rays", type=int, default=4096, help="train workload: rays per GPU per step (4096 = config c3, 65536 = c5)")
     ap.add_argument("--frames", type=int, default=0, help="c4 workload: number of camera poses (default 200)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="render workload: write the render outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 5 if args.impl == "reference" else 50
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "render"):
+        ap.error("--dump-outputs applies to the render workload of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

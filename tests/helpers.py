@@ -1,5 +1,9 @@
-"""Shared test fixtures: small synthetic scenes, rays, and the canonical form of the reference's sample stream."""
+"""Shared test fixtures: small synthetic scenes, rays, the canonical form of the reference's sample stream, and the
+recorded outputs the GPU parity tests compare with."""
 import functools
+import hashlib
+import os
+import zlib
 
 import numpy as np
 import torch
@@ -66,6 +70,76 @@ def bits_equal(a, b):
     if a.dtype.kind == "f":
         return np.array_equal(a.view(np.uint32 if a.itemsize == 4 else np.uint16), b.view(np.uint32 if b.itemsize == 4 else np.uint16))
     return np.array_equal(a, b)
+
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def _np(t):
+    return t.detach().cpu().numpy() if isinstance(t, torch.Tensor) else np.asarray(t)
+
+
+class Recorded:
+    """What one GPU parity test compares the product with, kept in tests/golden/recorded_<test module>.npz.
+
+    These tests used to run the reference's own CUDA kernels (oracle/_ref, compiled from the reference's sources, which are
+    not part of this repository) next to the product's on the same inputs.  The reference side is stored instead.  It was
+    recorded from this project's kernels at a commit where every one of these tests passed against the reference kernels,
+    so it is the reference's output bit for bit where a test asks for that, and within the test's tolerance elsewhere.
+
+    exact(name, t)   t must equal the recorded output bit for bit (stored as dtype, shape and SHA-256 of the bytes)
+    close(name, t)   t must match the recorded output within (rtol, atol) on a fixed sample of its elements: all of them
+                     for a small output, else `sample` seeded positions plus `sample` positions where it was non-zero
+    value(name, v)   the recorded value of a small array or scalar
+
+    With INERF_RECORD_GOLDEN=DIR set, the same calls store what they are given and the files are written to DIR when the
+    session ends."""
+
+    def __init__(self, store, prefix, record):
+        self.store, self.prefix, self.record = store, prefix, record
+
+    def _key(self, name):
+        return f"{self.prefix}::{name}"
+
+    def _get(self, name):
+        k = self._key(name)
+        if k not in self.store:
+            raise KeyError(f"{k} is not recorded under tests/golden (see helpers.Recorded)")
+        return self.store[k]
+
+    def exact(self, name, t):
+        a = np.ascontiguousarray(_np(t))
+        h = f"{a.dtype.str}{list(a.shape)}:{hashlib.sha256(a.tobytes()).hexdigest()}"
+        if self.record:
+            self.store[self._key(name)] = np.array(h)
+        else:
+            want = str(self._get(name))
+            assert h == want, f"{name}: differs from the recorded output ({h} vs {want})"
+
+    def close(self, name, t, rtol, atol, equal_nan=False, sample=128):
+        flat = _np(t).reshape(-1)
+        if self.record:
+            if flat.size <= 2 * sample:
+                idx = np.arange(flat.size)
+            else:
+                rng = np.random.RandomState(zlib.crc32(self._key(name).encode()))
+                nz = np.flatnonzero(flat)
+                idx = np.unique(np.concatenate([rng.choice(flat.size, sample, replace=False),
+                                                rng.choice(nz, min(sample, nz.size), replace=False)]))
+            self.store[self._key(name + "#shape")] = np.array(_np(t).shape, np.int64)
+            self.store[self._key(name + "#idx")] = idx.astype(np.int32 if flat.size < 2 ** 31 else np.int64)
+            self.store[self._key(name + "#val")] = flat[idx]
+            return
+        assert tuple(_np(t).shape) == tuple(self._get(name + "#shape")), name
+        idx = self._get(name + "#idx")
+        torch.testing.assert_close(torch.from_numpy(np.ascontiguousarray(flat[idx])), torch.from_numpy(self._get(name + "#val")),
+                                   rtol=rtol, atol=atol, equal_nan=equal_nan, msg=lambda m: f"{name}: {m}")
+
+    def value(self, name, v):
+        if self.record:
+            self.store[self._key(name)] = np.asarray(v)
+            return v
+        return self._get(name)
 
 
 def record_metric(name, **kv):

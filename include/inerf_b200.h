@@ -407,6 +407,34 @@ int inerf_adam_advance(float *step, const float *found_inf, void *stream);
 int inerf_project_labels(const float *rays_o, const float *rays_d, uint32_t N, const int32_t *labels, uint32_t nx, uint32_t ny,
                          uint32_t nz, const float *bbox_host, int32_t *out_label, float *out_t, void *stream);
 
+/* ---- volume extraction: the trained fields on a voxel grid ------------------------------------------------------------------
+ * The grid geometry and label convention of inerf_project_labels, so that an extracted label volume projects unchanged.
+ *
+ * Voxel (i,j,k) of an X x Y x Z grid over bbox (6 HOST floats: lo xyz, hi xyz) -> its point
+ *   p = lo + ((float)i / (float)X) * (hi - lo)        (per axis; fp32; one IEEE op each, in this order)
+ * = projection.voxel_points / grid_pts_coord, the cell centres inerf_project_labels walks.
+ * occupied (optional, u8 [X*Y*Z]): 1 where the point's occupancy cell is set in `bitfield` (NULL bitfield: all 1).  The cell
+ * is the one the marcher tests for a sample at p with dt = 0: cascade = clamped exponent of max|p|, then the cell of p in it.
+ * Every axis is 1..2048, X*Y*Z < 2^31, lo < hi on every axis and the bbox lies inside [-bound, bound]^3.
+ */
+int inerf_volume_points(const float *bbox_host, uint32_t X, uint32_t Y, uint32_t Z, const uint8_t *bitfield, uint32_t C,
+                        uint32_t H, float bound, float *xyzs, uint8_t *occupied, void *stream);
+
+size_t inerf_extract_scratch_ints(uint32_t X, uint32_t Y, uint32_t Z);
+/* The fields at every voxel, outputs C order [X,Y,Z](,3), each optional (at least one):
+ *   sigma  = density * desc->density_scale           (the sigma run_cuda composites and density_grid stores)
+ *   rgb    = colour for the single view direction view_dir_host (3 HOST floats; required iff rgb != NULL)
+ *   label  = 1 + argmax_k logits  if the voxel is live and sigma >= sigma_thresh, else 0
+ * Field values are bit-identical to inerf_field_forward at the voxel's point (d = view_dir), sigma multiplied by
+ * density_scale in fp32; the argmax runs over the fp16-rounded logits it stores, lowest index on ties.
+ * bitfield != NULL: a voxel whose occupancy cell is empty is NOT evaluated: sigma 0, rgb 0, label 0.
+ * bitfield == NULL: every voxel is evaluated.
+ * n_live (optional, device int32): number of voxels evaluated.  scratch: caller-owned, uninitialised,
+ * int32[inerf_extract_scratch_ints(X, Y, Z)]; required iff bitfield != NULL.  Every output element is written once. */
+int inerf_extract_volume(const inerf_field_desc *desc, const float *bbox_host, uint32_t X, uint32_t Y, uint32_t Z,
+                         const uint8_t *bitfield, uint32_t C, uint32_t H, const float *view_dir_host, float sigma_thresh,
+                         float *sigma, float *rgb, int32_t *label, int32_t *scratch, int32_t *n_live, void *stream);
+
 /* ---- frame finalisation (MaskTrainer.test / evaluate_one_epoch, nerf/utils.py:1425-1431, 1461-1485, 1624-1634) ----------------
  * rgb[N,3] / depth_u8[N] = (x * 255) truncated to uint8 (saturating), label[N] = argmax_k logits[N,K] (= the reference's
  * softmax + argmax; lowest index on ties; K <= 256).  depth / depth_u8 and logits / label may be NULL in pairs. */

@@ -1,7 +1,7 @@
 // Version / error-string entry points of libinerf_b200.
 #include "common.cuh"
 
-extern "C" int inerf_version(void) { return 1000; }
+extern "C" int inerf_version(void) { return 1001; }
 
 extern "C" const char* inerf_error_string(int code) {
     if (code > 0) return cudaGetErrorString((cudaError_t)code);

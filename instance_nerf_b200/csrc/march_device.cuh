@@ -35,6 +35,24 @@ __device__ __forceinline__ int clamped_exponent(float mx, int C) {
     return min(C - 1, max(0, e));
 }
 
+// Occupancy cell of point (x, y, z) at cascade `level` (raymarching.cu:1022-1033): the cell coordinates n (also returned,
+// with mip_bound = min(2^level, bound), for the DDA's exit test) and the bitfield index level * H^3 + morton(n).  Two latency
+// cuts that are exact: 1 / mip_bound is a power of two (exponent arithmetic) unless the cascade is clipped to `bound`
+// (precomputed quotient rbound), and the index is formed in integers whenever the reference's float expression is exact,
+// i.e. C * H^3 <= 2^24 (H3i != 0).  Shared by Walk::eval_cell and the volume extraction (field_fused.cu).
+__device__ __forceinline__ uint32_t cell_index(float x, float y, float z, int level, float bound, float rbound, float Hf, float Hm1,
+                                               uint32_t H3i, float H3, float& mip_bound, int& nx, int& ny, int& nz) {
+    const float pow2 = __uint_as_float((uint32_t)(127 + level) << 23);
+    const bool clipped = !(pow2 <= bound);   // fminf(2^level, bound) picks bound
+    mip_bound = clipped ? bound : pow2;
+    const float mip_rbound = clipped ? rbound : __uint_as_float((uint32_t)(127 - level) << 23);
+    const float hH = __fmul_rn(0.5f, Hf);
+    nx = (int)clampf(__fmul_rn(__fmaf_rn(x, mip_rbound, 1.0f), hH), 0.0f, Hm1);
+    ny = (int)clampf(__fmul_rn(__fmaf_rn(y, mip_rbound, 1.0f), hH), 0.0f, Hm1);
+    nz = (int)clampf(__fmul_rn(__fmaf_rn(z, mip_rbound, 1.0f), hH), 0.0f, Hm1);
+    return H3i ? (uint32_t)level * H3i + morton3D_enc(nx, ny, nz) : (uint32_t)__fmaf_rn((float)level, H3, (float)morton3D_enc(nx, ny, nz));
+}
+
 struct Walk {
     float ox, oy, oz, dx, dy, dz, rdx, rdy, rdz;
     float sx, sy, sz;  // 0.5 * sign(d)
@@ -117,9 +135,7 @@ struct Walk {
     // ONE cell evaluation of the DDA at parameter t (used by the render kernel's per-lane state machine).
     // Occupied: returns true with the sample (x, y, z, dt) and t advanced past it.  Empty: returns false with `tt` = the
     // parameter at which the ray leaves this cell; the caller then does `do { t += step_size(t); } while (t < tt);`.
-    // Same values as run() / the reference, with two latency cuts that are exact: 1 / mip_bound is a power of two (exponent
-    // arithmetic) unless the cascade is clipped to `bound` (precomputed quotient), and level * H^3 + morton is formed in
-    // integers whenever the reference's float expression (raymarching.cu:1033) is exact, i.e. C * H^3 <= 2^24.
+    // Same values as run() / the reference (the cell lookup is cell_index above).
     __device__ __forceinline__ bool eval_cell(float& t, float& x, float& y, float& z, float& dt, float& tt) {
         x = clampf(__fmaf_rn(t, dx, ox), -bound, bound);
         y = clampf(__fmaf_rn(t, dy, oy), -bound, bound);
@@ -128,16 +144,9 @@ struct Walk {
         const float mx = fmaxf(fabsf(x), fmaxf(fabsf(y), fabsf(z)));
         const float md = __fmul_rn(__fmul_rn(dt, Hf), 0.5f);
         const int level = max(clamped_exponent(mx, C), clamped_exponent(md, C));
-        const float pow2 = __uint_as_float((uint32_t)(127 + level) << 23);
-        const bool clipped = !(pow2 <= bound);   // fminf(2^level, bound) picks bound
-        const float mip_bound = clipped ? bound : pow2;
-        const float mip_rbound = clipped ? rbound : __uint_as_float((uint32_t)(127 - level) << 23);
-        const float hH = __fmul_rn(0.5f, Hf);
-        const int nx = (int)clampf(__fmul_rn(__fmaf_rn(x, mip_rbound, 1.0f), hH), 0.0f, Hm1);
-        const int ny = (int)clampf(__fmul_rn(__fmaf_rn(y, mip_rbound, 1.0f), hH), 0.0f, Hm1);
-        const int nz = (int)clampf(__fmul_rn(__fmaf_rn(z, mip_rbound, 1.0f), hH), 0.0f, Hm1);
-        const uint32_t index = H3i ? (uint32_t)level * H3i + morton3D_enc(nx, ny, nz)
-                                   : (uint32_t)__fmaf_rn((float)level, H3, (float)morton3D_enc(nx, ny, nz));
+        float mip_bound;
+        int nx, ny, nz;
+        const uint32_t index = cell_index(x, y, z, level, bound, rbound, Hf, Hm1, H3i, H3, mip_bound, nx, ny, nz);
         if (occupied_cached(index)) {
             t = __fadd_rn(t, dt);
             return true;

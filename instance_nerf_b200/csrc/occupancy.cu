@@ -269,6 +269,12 @@ int make_points(OccPoints* o, uint32_t C, uint32_t G, float bound, const int32_t
     fill_cascades(bound, C, G, o->scale, o->hgs, 1.0);
     return INERF_OK;
 }
+
+int scan_block_counts(int32_t* counts, uint32_t per_segment, uint32_t n_segments, int32_t* totals, cudaStream_t st) {
+    k_occ_scan<<<n_segments, 1024, 0, st>>>(counts, per_segment, totals);
+    INERF_LAUNCH_CHECK();
+    return INERF_OK;
+}
 }  // namespace occ
 
 extern "C" int inerf_occupancy_points(uint32_t C, uint32_t G, float bound, const int32_t* cells, uint32_t per_cascade, const float* noise,
@@ -308,8 +314,7 @@ extern "C" int inerf_occupancy_sample_cells(const float* density_grid, uint32_t 
     cudaStream_t st = (cudaStream_t)stream;
     k_occ_count<<<dim3(bpc, C), kOccBlock, 0, st>>>(density_grid, cpc, bpc, block_counts);
     INERF_LAUNCH_CHECK();
-    k_occ_scan<<<C, 1024, 0, st>>>(block_counts, bpc, n_occ);
-    INERF_LAUNCH_CHECK();
+    if (int e = occ::scan_block_counts(block_counts, bpc, C, n_occ, st)) return e;
     k_occ_compact<<<dim3(bpc, C), kOccBlock, 0, st>>>(density_grid, cpc, bpc, block_counts, occ_list);
     INERF_LAUNCH_CHECK();
     k_occ_pick<<<min(div_up((unsigned long long)C * N, 256), (unsigned int)(kNumSMs * 8)), 256, 0, st>>>(occ_list, n_occ, cpc, N, C, uniform_cells,

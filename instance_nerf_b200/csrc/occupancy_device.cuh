@@ -23,6 +23,10 @@ struct OccPoints {
 // fills `o` for C cascades of a G^3 grid (host side; defined in occupancy.cu); INERF_OK or an argument error
 int make_points(OccPoints* o, uint32_t C, uint32_t G, float bound, const int32_t* cells, uint32_t per_cascade, const float* noise, uint64_t seed);
 
+// exclusive scan, in place, of `n_segments` consecutive runs of `per_segment` int32 block counts; the total of segment s goes
+// to totals[s] (one launch on `st`, defined in occupancy.cu; also the compaction behind inerf_extract_volume)
+int scan_block_counts(int32_t* counts, uint32_t per_segment, uint32_t n_segments, int32_t* totals, cudaStream_t st);
+
 // splitmix64 finaliser over (seed, counter): 64 well-mixed bits per call, no state, no memory traffic
 __device__ __forceinline__ unsigned long long mix64(unsigned long long seed, unsigned long long counter) {
     unsigned long long z = seed + (counter + 1ull) * 0x9E3779B97F4A7C15ull;

@@ -140,6 +140,13 @@ class NeRFNetwork(NeRFRenderer):
     forward_fused = _InstanceNetwork.forward_fused
     _render_fused = _InstanceNetwork._render_fused
     _occupancy_density_fused = _InstanceNetwork._occupancy_density_fused
+    _extract_volume_fused = _InstanceNetwork._extract_volume_fused
+
+    def extract_volume(self, resolution, bbox=None, view_dir=None, sigma_thresh=None, skip_empty=True, labels=True, **kwargs):
+        """NeRFRenderer.extract_volume for sigma / rgb: this network has no instance head, so `labels` must be False."""
+        if labels:
+            raise ValueError("the stage-1 network has no instance head: call extract_volume(..., labels=False)")
+        return super().extract_volume(resolution, bbox, view_dir, sigma_thresh, skip_empty, labels=False, **kwargs)
 
     # ---- fused training (fp16 autocast, standard architecture): one launch forward, one launch backward -----------------
     def fused_train_available(self, x, d) -> bool:

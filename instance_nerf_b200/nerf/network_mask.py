@@ -254,6 +254,20 @@ class NeRFNetwork(NeRFMaskRenderer):
              ptr(tmp_grid), stream_ptr(tmp_grid.device))
         return True
 
+    def _extract_volume_fused(self, shape, bbox, bitfield, view_dir, sigma_thresh, sigma, rgb, label, n_live) -> bool:
+        """extract_volume as ONE launch (inerf_extract_volume; plus its occupancy pre-pass when `bitfield` is given): voxel ->
+        point -> hash encode -> sigma / colour / mask nets on tcgen05 -> sigma * density_scale, rgb, 1 + argmax label."""
+        if not self.fused_available():
+            return False
+        X, Y, Z = shape
+        dev = sigma.device
+        scratch = None if bitfield is None else torch.empty(int(lib().inerf_extract_scratch_ints(X, Y, Z)), dtype=torch.int32, device=dev)
+        desc = self._field_desc(self.density_scale)
+        call("inerf_extract_volume", ctypes.byref(desc), bbox.ctypes.data, X, Y, Z, ptr(bitfield), self.cascade, self.grid_size,
+             None if view_dir is None else view_dir.ctypes.data, float(sigma_thresh), ptr(sigma), ptr(rgb), ptr(label), ptr(scratch),
+             ptr(n_live), stream_ptr(dev))
+        return True
+
     # ---- reference operator sequence ----------------------------------------------------
     def _mlp(self, net, h):
         n = len(net)

@@ -432,6 +432,70 @@ class NeRFRenderer(nn.Module):
              ptr(mean), st)
         self._mean_density = mean
 
+    # -- volume extraction ------------------------------------------------------------------
+    def _extract_volume_fused(self, shape, bbox, bitfield, view_dir, sigma_thresh, sigma, rgb, label, n_live) -> bool:
+        """Hook: networks with the fused extraction kernel fill the outputs and return True (NeRFNetwork)."""
+        return False
+
+    @torch.no_grad()
+    def extract_volume(self, resolution, bbox=None, view_dir=None, sigma_thresh=None, skip_empty=True, labels=True, chunk=1 << 20):
+        """The trained fields on an X x Y x Z voxel grid over `bbox` (default `aabb_infer`; 6 floats lo xyz, hi xyz, inside
+        [-bound, bound]^3): voxel (i, j, k) sits at lo + (i, j, k) / (X, Y, Z) * (hi - lo), the geometry and label convention of
+        `projection.project_rays` / `project_masks`, so the label volume projects into any view unchanged.
+
+        -> {"sigma": float32 [X, Y, Z] (density * density_scale), "label": int32 [X, Y, Z] (1 + argmax of the instance logits
+        where sigma >= sigma_thresh, else 0; only with `labels`), "rgb": float32 [X, Y, Z, 3] (the colour seen along the unit
+        direction `view_dir`; only when it is given), "bbox": the 6 floats used, "n_live": device int32 [1], voxels evaluated}.
+
+        skip_empty (cuda_ray models): voxels whose occupancy cell is empty are not evaluated and come out 0 everywhere.
+        sigma_thresh: default min(mean_density, density_thresh), the threshold the occupancy bitfield was packed with.
+        Each of the two defaults costs one host read of a device value (aabb_infer, mean_density); a call that passes `bbox` and
+        `sigma_thresh` (host values) does not synchronise with the device.  One fused launch (plus an occupancy pre-pass) when the network has the fused field;
+        otherwise inerf_volume_points -> the network's forward under fp16 autocast in chunks of `chunk` voxels -> the same rules
+        in torch, on the GPU."""
+        X, Y, Z = (int(resolution),) * 3 if isinstance(resolution, int) else (int(r) for r in resolution)
+        bb = self.aabb_infer.tolist() if bbox is None else torch.as_tensor(bbox, dtype=torch.float32).reshape(6).tolist()
+        bb = tuple(float(v) for v in bb)
+        bb_host = np.ascontiguousarray(bb, dtype=np.float32)
+        vd = None if view_dir is None else np.ascontiguousarray(torch.as_tensor(view_dir, dtype=torch.float32).cpu().reshape(3).numpy())
+        gated = bool(skip_empty and self.cuda_ray)
+        if sigma_thresh is None:
+            sigma_thresh = min(float(self.mean_density), float(self.density_thresh)) if self.cuda_ray else float(self.density_thresh)
+        dev = self.aabb_infer.device
+        bitfield = self.density_bitfield if gated else None
+        sigma = torch.empty(X, Y, Z, dtype=torch.float32, device=dev)
+        rgb = torch.empty(X, Y, Z, 3, dtype=torch.float32, device=dev) if vd is not None else None
+        label = torch.empty(X, Y, Z, dtype=torch.int32, device=dev) if labels else None
+        n_live = torch.empty(1, dtype=torch.int32, device=dev)
+        if not self._extract_volume_fused((X, Y, Z), bb_host, bitfield, vd, float(sigma_thresh), sigma, rgb, label, n_live):
+            n = X * Y * Z
+            xyzs = torch.empty(n, 3, dtype=torch.float32, device=dev)
+            occupied = torch.empty(n, dtype=torch.uint8, device=dev)
+            call("inerf_volume_points", bb_host.ctypes.data, X, Y, Z, ptr(bitfield), self.cascade if gated else 0,
+                 self.grid_size if gated else 0, float(self.bound), ptr(xyzs), ptr(occupied), stream_ptr(dev))
+            live = occupied.bool()
+            d = torch.tensor([0.0, 0.0, 1.0] if vd is None else vd.tolist(), dtype=torch.float32, device=dev).expand(min(n, chunk), 3)
+            s_flat, c_flat = sigma.view(-1), None if rgb is None else rgb.view(-1, 3)
+            l_flat = None if label is None else label.view(-1)
+            for i in range(0, n, chunk):
+                j = min(n, i + chunk)
+                with torch.autocast("cuda", dtype=torch.float16):
+                    out = self(xyzs[i:j], d[:j - i])
+                s = out[0].float() * self.density_scale
+                s_flat[i:j] = torch.where(live[i:j], s, 0.0)
+                if c_flat is not None:
+                    c_flat[i:j] = torch.where(live[i:j, None], out[1].float(), 0.0)
+                if l_flat is not None:
+                    arg = torch.argmax(out[2], dim=-1).to(torch.int32) + 1
+                    l_flat[i:j] = torch.where(live[i:j] & (s >= sigma_thresh), arg, 0)
+            n_live.copy_(live.sum().view(1))
+        out = {"sigma": sigma, "bbox": bb, "n_live": n_live}
+        if label is not None:
+            out["label"] = label
+        if rgb is not None:
+            out["rgb"] = rgb
+        return out
+
     # -- entry point (mask_renderer.py:551-589) ------------------------------------------
     def render(self, rays_o, rays_d, staged=False, max_ray_batch=4096, render_mask=False, **kwargs):
         _run = self.run_cuda if self.cuda_ray else self.run

@@ -435,6 +435,29 @@ int inerf_extract_volume(const inerf_field_desc *desc, const float *bbox_host, u
                          const uint8_t *bitfield, uint32_t C, uint32_t H, const float *view_dir_host, float sigma_thresh,
                          float *sigma, float *rgb, int32_t *label, int32_t *scratch, int32_t *n_live, void *stream);
 
+/* ---- mesh export: marching cubes over a float volume ------------------------------------------------------------------------
+ * v: device float [X,Y,Z] in C order, sample (i,j,k) at the voxel point of inerf_volume_points:
+ *   p = lo + ((float)i / (float)X) * (hi - lo)        (per axis; bbox_host = 6 HOST floats lo xyz, hi xyz; finite, lo < hi)
+ * Inside means v > iso (NaN: outside).  The table (csrc/mc_table.h, generated by scripts/gen_mc_table.py) cuts every run of
+ * inside corners on a cube face off by its own segment, so neighbouring cubes agree and the surface is closed where it does
+ * not reach the volume's border; triangle normals (right-hand rule) point toward v < iso.
+ *   vertices   one per lattice edge whose two samples differ in inside-ness, owned by its lower sample; ordered by that
+ *              sample's C-order index, then by axis (x, y, z).  Along the edge's axis the vertex sits at s = (float)i + t,
+ *              t = fminf(fmaxf((iso - va) / (vb - va), 0), 1), world coordinate lo + (s / (float)X) * (hi - lo); the other two
+ *              coordinates are the sample's own.  fp32, one IEEE op each, in this order (a vertex with t = 0 is the voxel
+ *              point bit for bit; the clamp gives a NaN sample the lower end).
+ *   triangles  int32 [F,3] vertex indices, ordered by cube (C order of its lower corner) and then by table order.
+ * Every output position is a prefix sum over C order (no atomics): the same bytes on every run.
+ * Every axis is 2..2048, X*Y*Z < 2^31, and 3*X*Y*Z and 5*(X-1)*(Y-1)*(Z-1) (the most vertices / triangles a volume can
+ * yield) < 2^31, so that every index and count fits int32.
+ * Two calls: inerf_mesh_count leaves (V, F) in counts[2] (device int32) and its per-sample state in scratch (caller-owned,
+ * uninitialised, int32[inerf_mesh_scratch_ints(X, Y, Z)]; 0 = sizes out of range); the caller sizes verts float [V,3] and
+ * tris int32 [F,3] and calls inerf_mesh_emit with the same v, sizes, iso and scratch (F == 0: nothing to emit). */
+size_t inerf_mesh_scratch_ints(uint32_t X, uint32_t Y, uint32_t Z);
+int inerf_mesh_count(const float *v, uint32_t X, uint32_t Y, uint32_t Z, float iso, int32_t *scratch, int32_t *counts, void *stream);
+int inerf_mesh_emit(const float *v, uint32_t X, uint32_t Y, uint32_t Z, const float *bbox_host, float iso, int32_t *scratch,
+                    float *verts, int32_t *tris, void *stream);
+
 /* ---- frame finalisation (MaskTrainer.test / evaluate_one_epoch, nerf/utils.py:1425-1431, 1461-1485, 1624-1634) ----------------
  * rgb[N,3] / depth_u8[N] = (x * 255) truncated to uint8 (saturating), label[N] = argmax_k logits[N,K] (= the reference's
  * softmax + argmax; lowest index on ties; K <= 256).  depth / depth_u8 and logits / label may be NULL in pairs. */

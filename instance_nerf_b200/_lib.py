@@ -115,6 +115,8 @@ _PROTOS = {
     "inerf_render_fused_perturb": [POINTER(FieldDesc), _P, _P, _P, _P, _P, _P, _U, _U, _U, _F, _U, _F, _P, _P, _P, _P, _P, _P],
     "inerf_volume_points": [_P, _U, _U, _U, _P, _U, _U, _F, _P, _P, _P],
     "inerf_extract_volume": [POINTER(FieldDesc), _P, _U, _U, _U, _P, _U, _U, _P, _F, _P, _P, _P, _P, _P, _P],
+    "inerf_mesh_count": [_P, _U, _U, _U, _F, _P, _P, _P],
+    "inerf_mesh_emit": [_P, _U, _U, _U, _P, _F, _P, _P, _P, _P],
 }
 _SPECIAL = {
     "inerf_version": ([], c_int),
@@ -125,6 +127,7 @@ _SPECIAL = {
     "inerf_march_scratch_floats": ([_U, _U], c_size_t),
     "inerf_occupancy_sample_scratch_ints": ([_U, _U], c_size_t),
     "inerf_extract_scratch_ints": ([_U, _U, _U], c_size_t),
+    "inerf_mesh_scratch_ints": ([_U, _U, _U], c_size_t),
 }
 
 # Every symbol include/inerf_b200.h declares; tests check the .so exports all of them.

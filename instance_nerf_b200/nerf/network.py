@@ -148,6 +148,12 @@ class NeRFNetwork(NeRFRenderer):
             raise ValueError("the stage-1 network has no instance head: call extract_volume(..., labels=False)")
         return super().extract_volume(resolution, bbox, view_dir, sigma_thresh, skip_empty, labels=False, **kwargs)
 
+    def extract_mesh(self, resolution=256, bbox=None, threshold=10, view_dir=None, labels=True, skip_empty=True):
+        """NeRFRenderer.extract_mesh with vertex colours only: this network has no instance head, so `labels` must be False."""
+        if labels:
+            raise ValueError("the stage-1 network has no instance head: call extract_mesh(..., labels=False)")
+        return super().extract_mesh(resolution, bbox, threshold, view_dir, labels=False, skip_empty=skip_empty)
+
     # ---- fused training (fp16 autocast, standard architecture): one launch forward, one launch backward -----------------
     def fused_train_available(self, x, d) -> bool:
         if not (self.fused_available() and x.is_cuda and torch.is_autocast_enabled() and not x.requires_grad and not d.requires_grad):

@@ -496,6 +496,46 @@ class NeRFRenderer(nn.Module):
             out["rgb"] = rgb
         return out
 
+    @torch.no_grad()
+    def extract_mesh(self, resolution=256, bbox=None, threshold=10, view_dir=None, labels=True, skip_empty=True):
+        """A triangle mesh of the density surface, with the fields at its vertices: extract_volume's sigma on the voxel grid
+        -> marching cubes at iso = threshold * density_scale (the reference's save_mesh threshold applies to the density
+        before density_scale; extract_volume's sigma includes it) -> the field at every vertex.
+
+        -> {"verts": float32 [V, 3], "faces": int32 [F, 3] (normals toward low density), "bbox", "iso",
+        "rgb": float32 [V, 3] (colour seen along `view_dir`; only when it is given),
+        "vertex_label": int32 [V] (1 + argmax of the instance logits, lowest index on ties) and "face_label": int32 [F]
+        (majority of the face's vertex labels, the smallest when all three differ); both only with `labels`}.
+
+        The vertex fields come from the fused field forward when the network has it, else from the network's forward under
+        fp16 autocast.  A call that passes `bbox` reads the device once (the mesh size)."""
+        vol = self.extract_volume(resolution, bbox=bbox, sigma_thresh=0.0, skip_empty=skip_empty, labels=False)
+        iso = float(threshold) * float(self.density_scale)
+        from ..mesh import face_labels, mesh_from_volume
+        out = mesh_from_volume(vol["sigma"], vol["bbox"], iso)
+        out.update(bbox=vol["bbox"], iso=iso)
+        if view_dir is None and not labels:
+            return out
+        verts = out["verts"]
+        d = torch.empty_like(verts)
+        for a, c in enumerate((0.0, 0.0, 1.0) if view_dir is None else torch.as_tensor(view_dir, dtype=torch.float32).reshape(3).tolist()):
+            d[:, a] = float(c)
+        if verts.shape[0] == 0:
+            rgb, logits = torch.empty_like(verts), torch.empty(0, 1, device=verts.device)
+        elif self.fused_available():
+            _, rgb, logits = self.forward_fused(verts, d, want_masks=labels)
+        else:
+            with torch.autocast("cuda", dtype=torch.float16):
+                f = self(verts, d)
+            rgb, logits = f[1].float(), f[2] if labels else None
+        if view_dir is not None:
+            out["rgb"] = rgb
+        if labels:
+            vl = torch.argmax(logits, dim=-1).to(torch.int32) + 1
+            out["vertex_label"] = vl
+            out["face_label"] = face_labels(vl, out["faces"])
+        return out
+
     # -- entry point (mask_renderer.py:551-589) ------------------------------------------
     def render(self, rays_o, rays_d, staged=False, max_ray_batch=4096, render_mask=False, **kwargs):
         _run = self.run_cuda if self.cuda_ray else self.run

@@ -491,4 +491,16 @@ __device__ __forceinline__ void load_weights(uint8_t* smem, uint32_t w_off, cons
 
 int validate(const inerf_field_desc* d);
 
+// Host: launch a persistent field kernel -- one CTA per SM, or one per tile when there are fewer tiles of `rows` -- with `smem`
+// bytes of dynamic shared memory.  The attribute is per device and cheap to set, so every launch sets it.
+template <typename... P, typename... A>
+inline int launch_persistent(void (*kernel)(P...), uint32_t rows, uint32_t threads, uint32_t smem, cudaStream_t stream, A... args) {
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    const uint32_t num_tiles = (rows + kTile - 1) / kTile, sms = (uint32_t)device_sm_count();
+    kernel<<<num_tiles < sms ? num_tiles : sms, threads, smem, stream>>>(args...);
+    INERF_LAUNCH_CHECK();
+    return INERF_OK;
+}
+
 }  // namespace field

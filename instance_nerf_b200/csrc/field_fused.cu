@@ -18,8 +18,7 @@ using namespace field;
 // ---- gather and MLP chain as concurrent roles of ONE CTA per SM -----------------------------------------------------------
 // The structure is the render kernel's (render_fused.cu) without its marcher and compositor: 16 gather warps (thread = sample
 // row x 4 of the 16 levels, 64 registers) fill one of two operand stages while 8 chain warps (96 registers) run the tcgen05
-// chain of the previous tile and write sigma / rgb / logits (and the saved mask-net input row); the gather warps never wait
-// for an epilogue.
+// chain of the previous tile and store its results; the gather warps never wait for an epilogue.
 constexpr uint32_t kWsChainT = 256, kWsGatherT = 512, kWsThreads = kWsChainT + kWsGatherT, kWsStages = 2;
 
 struct WsCtrl {
@@ -34,137 +33,17 @@ struct WsSmem {
     static __host__ __device__ uint32_t bytes(uint32_t K) { return ctrl(K) + (uint32_t)sizeof(WsCtrl) + 16u; }
 };
 
-__global__ void __launch_bounds__(kWsThreads, 1) k_field_forward_ws(inerf_field_desc desc, const float* __restrict__ xyzs,
-                                                                    const float* __restrict__ dirs, uint32_t B_rows,
-                                                                    float* __restrict__ sigmas, float* __restrict__ rgbs,
-                                                                    float* __restrict__ masks, uint4* __restrict__ x0_save,
-                                                                    uint4* __restrict__ xs_save) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const uint32_t K = desc.K, Kp = weight_layout(K).Kp;
-    WsCtrl* ctl = reinterpret_cast<WsCtrl*>(smem + WsSmem::ctrl(K));
-    const uint32_t tid = threadIdx.x;
-    load_weights(smem, WsSmem::W, desc.weights, K);
-    init_levels(ctl->lg, desc.offsets, desc.L, desc.S, desc.H, tid);
-    if (tid == 0) {
-        for (uint32_t i = 0; i < kWsStages; i++) { umma::mbar_init(&ctl->a_full[i], kWsGatherT / 32); umma::mbar_init(&ctl->a_empty[i], 1); }
-        umma::mbar_init(&ctl->mma_bar, 1);
-        umma::mbar_fence_init();
-    }
-    if (tid < 32) umma::tmem_alloc<kTmemCols>(&ctl->tmem_slot);
-    umma::fence_async_smem();
-    umma::fence_before_sync();
-    __syncthreads();
-    umma::fence_after_sync();
-    const uint32_t tmem_base = ctl->tmem_slot;
-    const uint32_t B = desc.n_valid ? min(B_rows, (uint32_t)max(0, __ldg(desc.n_valid))) : B_rows;   // rows past *n_valid: padding
-    const uint32_t num_tiles = (B + kTile - 1) / kTile;
-    const bool with_masks = masks != nullptr;
-
-    if (tid < kWsChainT) {
-        // ------------------------------------------------------------------------------------------------ chain --
-        umma::reg_alloc<96>();
-        const uint32_t warp = tid >> 5, lane = tid & 31;
-        uint32_t phase = 0, it = 0;
-        auto chain_sync = [] { umma::named_sync<1, kWsChainT>(); };
-        for (uint32_t tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, it++) {
-            const uint32_t sa = it % kWsStages;
-            umma::mbar_wait(&ctl->a_full[sa], (it / kWsStages) & 1u);
-            const uint32_t a_es = WsSmem::A + sa * kStageBytes;
-            const ChainBufs bufs{a_es, a_es + kBytesEs, a_es + kBytesEs + kBytesCi, WsSmem::W};
-            const uint32_t orow = tile * kTile + (warp & 3u) * 32u + lane;
-            const float sigma = mlp_chain(smem, bufs, tmem_base, &ctl->mma_bar, phase, K, desc.density_scale, with_masks, tid, &ctl->a_empty[sa],
-                                          chain_sync, [&](float) {
-                // training: keep the mask-net input row (32 mask-table features | 15 geo | 0, fp16) for the backward pass.  The row's
-                // owner wrote the geo columns itself a moment ago, and the stage is only released after the layer-0 MMAs.
-                if (x0_save != nullptr && warp < 4 && orow < B) {
-#pragma unroll
-                    for (uint32_t c = 0; c < 6; c++)
-                        x0_save[(size_t)orow * 6 + c] =
-                            *reinterpret_cast<const uint4*>(smem + bufs.a_mi + umma::tile_off(tid, c * 8, kLBO, sbo_of(48)));
-                }
-                // stage-1 training: keep the inputs of BOTH nets -- 32 sigma-table features | SH16, geo15, 0 (fp16 [.,64])
-                if (xs_save != nullptr && warp < 4 && orow < B) {
-#pragma unroll
-                    for (uint32_t c = 0; c < 4; c++) {
-                        xs_save[(size_t)orow * 8 + c] = *reinterpret_cast<const uint4*>(smem + bufs.a_es + umma::tile_off(tid, c * 8, kLBO, sbo_of(32)));
-                        xs_save[(size_t)orow * 8 + 4 + c] = *reinterpret_cast<const uint4*>(smem + bufs.a_ci + umma::tile_off(tid, c * 8, kLBO, sbo_of(32)));
-                    }
-                }
-            });
-            if (warp < 4) {
-                float rgb[3];
-                epilogue_rgb(tmem_base, rgb, tid);
-                if (orow < B) {
-                    sigmas[orow] = sigma;
-                    rgbs[(size_t)orow * 3] = rgb[0]; rgbs[(size_t)orow * 3 + 1] = rgb[1]; rgbs[(size_t)orow * 3 + 2] = rgb[2];
-                }
-            }
-            if (with_masks) {
-                const uint32_t chunks = Kp / 16, c_begin = (warp >> 2) ? (chunks + 1) / 2 : 0, c_end = (warp >> 2) ? chunks : (chunks + 1) / 2;
-                for (uint32_t c = c_begin; c < c_end; c++) {
-                    uint32_t v[16];
-                    umma::tmem_ld16(tmem_base + D_d + (((warp & 3u) * 32u) << 16) + c * 16, v);
-                    umma::tmem_ld_wait();
-                    if (orow < B) {
-                        float* out = masks + (size_t)orow * K + c * 16;
-                        if ((K & 3u) == 0 && c * 16 + 16 <= K) {
-#pragma unroll
-                            for (int i = 0; i < 4; i++)
-                                reinterpret_cast<float4*>(out)[i] = make_float4(__half2float(__float2half_rn(__uint_as_float(v[4 * i]))),
-                                                                                __half2float(__float2half_rn(__uint_as_float(v[4 * i + 1]))),
-                                                                                __half2float(__float2half_rn(__uint_as_float(v[4 * i + 2]))),
-                                                                                __half2float(__float2half_rn(__uint_as_float(v[4 * i + 3]))));
-                        } else {
-#pragma unroll
-                            for (int i = 0; i < 16; i++)
-                                if (c * 16 + i < K) out[i] = __half2float(__float2half_rn(__uint_as_float(v[i])));
-                        }
-                    }
-                }
-            }
-            umma::fence_before_sync();
-            chain_sync();   // TMEM and the chain's hidden tiles are reused by the next tile
-        }
-    } else {
-        // ----------------------------------------------------------------------------------------------- gather --
-        umma::reg_dealloc<64>();
-        const uint32_t gt = tid - kWsChainT, row = gt & (kTile - 1), quarter = gt >> 7;
-        const float inv2b = __fdiv_rn(1.0f, __fmul_rn(2.0f, desc.bound));
-        const uint2* table = reinterpret_cast<const uint2*>(desc.table_packed);
-        uint32_t it = 0;
-        for (uint32_t tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, it++) {
-            const uint32_t sa = it % kWsStages;
-            if (it >= kWsStages) umma::mbar_wait(&ctl->a_empty[sa], ((it / kWsStages) - 1u) & 1u);
-            const uint32_t s = tile * kTile + row;
-            if (s < B) {   // rows past the end keep stale operands: their outputs are never stored
-                const uint32_t a_es = WsSmem::A + sa * kStageBytes, a_ci = a_es + kBytesEs, a_mi = a_ci + kBytesCi;
-                float x01[3];
-                bool oob = false;
-#pragma unroll
-                for (int d = 0; d < 3; d++) {
-                    x01[d] = __fmul_rn(__fadd_rn(__ldg(xyzs + (size_t)s * 3 + d), desc.bound), inv2b);  // grid.py:149
-                    oob |= (x01[d] < 0.f || x01[d] > 1.f);
-                }
-                if (quarter == 0) sh16_to_smem(__ldg(dirs + (size_t)s * 3), __ldg(dirs + (size_t)s * 3 + 1), __ldg(dirs + (size_t)s * 3 + 2), smem, a_ci, row);
-                encode4(x01, oob, quarter * 4, ctl->lg, table, smem, a_es, a_mi, row);
-            }
-            umma::fence_async_smem();
-            __syncwarp();
-            if ((gt & 31u) == 0) umma::mbar_arrive(&ctl->a_full[sa]);   // one arrival per gather warp
-        }
-    }
-    umma::fence_before_sync();
-    __syncthreads();
-    if (tid < 32) umma::tmem_dealloc<kTmemCols>(tmem_base);
-}
-
-// ---- occupancy-grid density sweep (update_extra_state, nerf/mask_renderer.py:466-527) ------------------------------------
-// tmp_grid[c, cell] = density(jittered point of the cell) * density_scale for every sample of the sweep, in ONE launch with
-// the role structure above: the gather warps make each point from its cell id (Morton decode, cascade scale, jitter --
-// occupancy_device.cuh) instead of reading a sample stream, the chain warps run the sigma-net only and scatter the result to
-// the cell.  The reference goes through meshgrid / morton3D / rand_like / two table casts / encode / 2 GEMMs / index_put per
-// (block, cascade) from 5 nested Python loops.
-__global__ void __launch_bounds__(kWsThreads, 1) k_occupancy_density(inerf_field_desc desc, occ::OccPoints pts, uint32_t n, float* __restrict__ tmp_grid) {
+// The CTA of the three per-sample field kernels (k_field_forward_ws, k_occupancy_density, k_extract_volume).  What differs
+// between them is a Job:
+//   rows(desc)                  the number of rows, read once per CTA
+//   point(s, p)                 gather warps: the point of row s < rows
+//   sh_row(s, smem, a_ci, row)  gather warps: the SH16 columns of the colour-net input of row s (nothing for density only)
+//   tile(...)                   chain warps: the chain over one gathered stage (mlp_chain or sigma_chain, which releases the
+//                               stage), then the stores of rows row0 .. row0 + 127 below n
+// A parameter struct that a job indexes at run time (OccPoints' per-cascade arrays) is a __grid_constant__ kernel parameter held
+// by reference: a copy inside the job would go to local memory.
+template <typename Job>
+__device__ __forceinline__ void ws_field_cta(const inerf_field_desc desc, const Job& job) {
     extern __shared__ __align__(1024) uint8_t smem[];
     const uint32_t K = desc.K;
     WsCtrl* ctl = reinterpret_cast<WsCtrl*>(smem + WsSmem::ctrl(K));
@@ -182,9 +61,11 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_occupancy_density(inerf_field
     __syncthreads();
     umma::fence_after_sync();
     const uint32_t tmem_base = ctl->tmem_slot;
+    const uint32_t n = job.rows(desc);
     const uint32_t num_tiles = (n + kTile - 1) / kTile;
 
     if (tid < kWsChainT) {
+        // ------------------------------------------------------------------------------------------------ chain --
         umma::reg_alloc<96>();
         uint32_t phase = 0, it = 0;
         auto chain_sync = [] { umma::named_sync<1, kWsChainT>(); };
@@ -193,17 +74,12 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_occupancy_density(inerf_field
             umma::mbar_wait(&ctl->a_full[sa], (it / kWsStages) & 1u);
             const uint32_t a_es = WsSmem::A + sa * kStageBytes;
             const ChainBufs bufs{a_es, a_es + kBytesEs, a_es + kBytesEs + kBytesCi, WsSmem::W};
-            const float sigma = sigma_chain(smem, bufs, tmem_base, &ctl->mma_bar, phase, K, tid, &ctl->a_empty[sa], chain_sync);
-            const uint32_t s = tile * kTile + tid;
-            if (tid < kTile && s < n) {
-                const uint32_t c = s / pts.per_cascade;
-                const uint32_t m = pts.cells ? (uint32_t)__ldg(pts.cells + s) : s - c * pts.per_cascade;
-                tmp_grid[(size_t)c * pts.G * pts.G * pts.G + m] = __fmul_rn(sigma, desc.density_scale);   // `sigmas *= self.density_scale`
-            }
+            job.tile(desc, smem, bufs, tmem_base, &ctl->mma_bar, phase, &ctl->a_empty[sa], chain_sync, tile * kTile, n, tid);
             umma::fence_before_sync();
-            chain_sync();   // TMEM and the hidden tile are reused by the next tile
+            chain_sync();   // TMEM and the chain's hidden tiles are reused by the next tile
         }
     } else {
+        // ----------------------------------------------------------------------------------------------- gather --
         umma::reg_dealloc<64>();
         const uint32_t gt = tid - kWsChainT, row = gt & (kTile - 1), quarter = gt >> 7;
         const float inv2b = __fdiv_rn(1.0f, __fmul_rn(2.0f, desc.bound));
@@ -213,17 +89,17 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_occupancy_density(inerf_field
             const uint32_t sa = it % kWsStages;
             if (it >= kWsStages) umma::mbar_wait(&ctl->a_empty[sa], ((it / kWsStages) - 1u) & 1u);
             const uint32_t s = tile * kTile + row;
-            if (s < n) {
-                const uint32_t a_es = WsSmem::A + sa * kStageBytes, a_mi = a_es + kBytesEs + kBytesCi;
-                float xyz[3], x01[3];
-                uint32_t flat;
-                occ::occ_point(pts, s, xyz, flat);
+            if (s < n) {   // rows past the end keep stale operands: their outputs are never stored
+                const uint32_t a_es = WsSmem::A + sa * kStageBytes, a_ci = a_es + kBytesEs, a_mi = a_ci + kBytesCi;
+                float p[3], x01[3];
+                job.point(s, p);
                 bool oob = false;
 #pragma unroll
                 for (int d = 0; d < 3; d++) {
-                    x01[d] = __fmul_rn(__fadd_rn(xyz[d], desc.bound), inv2b);  // grid.py:149
+                    x01[d] = __fmul_rn(__fadd_rn(p[d], desc.bound), inv2b);  // grid.py:149
                     oob |= (x01[d] < 0.f || x01[d] > 1.f);
                 }
+                if (quarter == 0) job.sh_row(s, smem, a_ci, row);
                 encode4(x01, oob, quarter * 4, ctl->lg, table, smem, a_es, a_mi, row);
             }
             umma::fence_async_smem();
@@ -234,6 +110,128 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_occupancy_density(inerf_field
     umma::fence_before_sync();
     __syncthreads();
     if (tid < 32) umma::tmem_dealloc<kTmemCols>(tmem_base);
+}
+
+// ---- field forward: a sample stream (xyzs, dirs) -> sigma / rgb / logits, and for training the saved net inputs -------------
+struct ForwardJob {
+    const float* xyzs;
+    const float* dirs;
+    uint32_t B_rows;
+    float* sigmas;
+    float* rgbs;
+    float* masks;
+    uint4* x0_save;
+    uint4* xs_save;
+
+    __device__ __forceinline__ uint32_t rows(const inerf_field_desc& desc) const {   // rows past *n_valid: padding
+        return desc.n_valid ? min(B_rows, (uint32_t)max(0, __ldg(desc.n_valid))) : B_rows;
+    }
+    __device__ __forceinline__ void point(uint32_t s, float p[3]) const {
+#pragma unroll
+        for (int d = 0; d < 3; d++) p[d] = __ldg(xyzs + (size_t)s * 3 + d);
+    }
+    __device__ __forceinline__ void sh_row(uint32_t s, uint8_t* smem, uint32_t a_ci, uint32_t row) const {
+        sh16_to_smem(__ldg(dirs + (size_t)s * 3), __ldg(dirs + (size_t)s * 3 + 1), __ldg(dirs + (size_t)s * 3 + 2), smem, a_ci, row);
+    }
+    template <typename Sync>
+    __device__ __forceinline__ void tile(const inerf_field_desc& desc, uint8_t* smem, const ChainBufs& bufs, uint32_t tmem_base, uint64_t* mma_bar,
+                                         uint32_t& phase, uint64_t* release, Sync&& chain_sync, uint32_t row0, uint32_t B, uint32_t tid) const {
+        const uint32_t K = desc.K, Kp = weight_layout(K).Kp;
+        const uint32_t warp = tid >> 5, lane = tid & 31;
+        const bool with_masks = masks != nullptr;
+        const uint32_t orow = row0 + (warp & 3u) * 32u + lane;
+        const float sigma = mlp_chain(smem, bufs, tmem_base, mma_bar, phase, K, desc.density_scale, with_masks, tid, release, chain_sync, [&](float) {
+            // training: keep the mask-net input row (32 mask-table features | 15 geo | 0, fp16) for the backward pass.  The row's
+            // owner wrote the geo columns itself a moment ago, and the stage is only released after the layer-0 MMAs.
+            if (x0_save != nullptr && warp < 4 && orow < B) {
+#pragma unroll
+                for (uint32_t c = 0; c < 6; c++)
+                    x0_save[(size_t)orow * 6 + c] = *reinterpret_cast<const uint4*>(smem + bufs.a_mi + umma::tile_off(tid, c * 8, kLBO, sbo_of(48)));
+            }
+            // stage-1 training: keep the inputs of BOTH nets -- 32 sigma-table features | SH16, geo15, 0 (fp16 [.,64])
+            if (xs_save != nullptr && warp < 4 && orow < B) {
+#pragma unroll
+                for (uint32_t c = 0; c < 4; c++) {
+                    xs_save[(size_t)orow * 8 + c] = *reinterpret_cast<const uint4*>(smem + bufs.a_es + umma::tile_off(tid, c * 8, kLBO, sbo_of(32)));
+                    xs_save[(size_t)orow * 8 + 4 + c] = *reinterpret_cast<const uint4*>(smem + bufs.a_ci + umma::tile_off(tid, c * 8, kLBO, sbo_of(32)));
+                }
+            }
+        });
+        if (warp < 4) {
+            float rgb[3];
+            epilogue_rgb(tmem_base, rgb, tid);
+            if (orow < B) {
+                sigmas[orow] = sigma;
+                rgbs[(size_t)orow * 3] = rgb[0]; rgbs[(size_t)orow * 3 + 1] = rgb[1]; rgbs[(size_t)orow * 3 + 2] = rgb[2];
+            }
+        }
+        if (with_masks) {
+            const uint32_t chunks = Kp / 16, c_begin = (warp >> 2) ? (chunks + 1) / 2 : 0, c_end = (warp >> 2) ? chunks : (chunks + 1) / 2;
+            for (uint32_t c = c_begin; c < c_end; c++) {
+                uint32_t v[16];
+                umma::tmem_ld16(tmem_base + D_d + (((warp & 3u) * 32u) << 16) + c * 16, v);
+                umma::tmem_ld_wait();
+                if (orow < B) {
+                    float* out = masks + (size_t)orow * K + c * 16;
+                    if ((K & 3u) == 0 && c * 16 + 16 <= K) {
+#pragma unroll
+                        for (int i = 0; i < 4; i++)
+                            reinterpret_cast<float4*>(out)[i] = make_float4(__half2float(__float2half_rn(__uint_as_float(v[4 * i]))),
+                                                                            __half2float(__float2half_rn(__uint_as_float(v[4 * i + 1]))),
+                                                                            __half2float(__float2half_rn(__uint_as_float(v[4 * i + 2]))),
+                                                                            __half2float(__float2half_rn(__uint_as_float(v[4 * i + 3]))));
+                    } else {
+#pragma unroll
+                        for (int i = 0; i < 16; i++)
+                            if (c * 16 + i < K) out[i] = __half2float(__float2half_rn(__uint_as_float(v[i])));
+                    }
+                }
+            }
+        }
+    }
+};
+
+__global__ void __launch_bounds__(kWsThreads, 1) k_field_forward_ws(inerf_field_desc desc, const float* __restrict__ xyzs,
+                                                                    const float* __restrict__ dirs, uint32_t B_rows,
+                                                                    float* __restrict__ sigmas, float* __restrict__ rgbs,
+                                                                    float* __restrict__ masks, uint4* __restrict__ x0_save,
+                                                                    uint4* __restrict__ xs_save) {
+    ws_field_cta(desc, ForwardJob{xyzs, dirs, B_rows, sigmas, rgbs, masks, x0_save, xs_save});
+}
+
+// ---- occupancy-grid density sweep (update_extra_state, nerf/mask_renderer.py:466-527) ------------------------------------
+// tmp_grid[c, cell] = density(jittered point of the cell) * density_scale for every sample of the sweep, in ONE launch with
+// the role structure above: the gather warps make each point from its cell id (Morton decode, cascade scale, jitter --
+// occupancy_device.cuh) instead of reading a sample stream, the chain warps run the sigma-net only and scatter the result to
+// the cell.  The reference goes through meshgrid / morton3D / rand_like / two table casts / encode / 2 GEMMs / index_put per
+// (block, cascade) from 5 nested Python loops.
+struct OccJob {
+    const occ::OccPoints& pts;
+    uint32_t n;
+    float* tmp_grid;
+
+    __device__ __forceinline__ uint32_t rows(const inerf_field_desc&) const { return n; }
+    __device__ __forceinline__ void point(uint32_t s, float p[3]) const {
+        uint32_t flat;
+        occ::occ_point(pts, s, p, flat);
+    }
+    __device__ __forceinline__ void sh_row(uint32_t, uint8_t*, uint32_t, uint32_t) const {}
+    template <typename Sync>
+    __device__ __forceinline__ void tile(const inerf_field_desc& desc, uint8_t* smem, const ChainBufs& bufs, uint32_t tmem_base, uint64_t* mma_bar,
+                                         uint32_t& phase, uint64_t* release, Sync&& chain_sync, uint32_t row0, uint32_t, uint32_t tid) const {
+        const float sigma = sigma_chain(smem, bufs, tmem_base, mma_bar, phase, desc.K, tid, release, chain_sync);
+        const uint32_t s = row0 + tid;
+        if (tid < kTile && s < n) {
+            const uint32_t c = s / pts.per_cascade;
+            const uint32_t m = pts.cells ? (uint32_t)__ldg(pts.cells + s) : s - c * pts.per_cascade;
+            tmp_grid[(size_t)c * pts.G * pts.G * pts.G + m] = __fmul_rn(sigma, desc.density_scale);   // `sigmas *= self.density_scale`
+        }
+    }
+};
+
+__global__ void __launch_bounds__(kWsThreads, 1) k_occupancy_density(inerf_field_desc desc, const __grid_constant__ occ::OccPoints pts, uint32_t n,
+                                                                     float* __restrict__ tmp_grid) {
+    ws_field_cta(desc, OccJob{pts, n, tmp_grid});
 }
 
 // ---- volume extraction (inerf_volume_points / inerf_extract_volume) ---------------------------------------------------------
@@ -330,113 +328,75 @@ __global__ void __launch_bounds__(kVolBlock) k_vol_compact(VolGeom g, const int3
     }
 }
 
-// The fused extraction: k_occupancy_density's role structure with a voxel front and an argmax epilogue.  The gather warps turn
-// row s of the tile loop into a voxel (live_ids[s], or voxel s when every voxel is evaluated) and its point, and
-// gather both tables and the SH row of the one view direction; the chain warps run the full mlp_chain (mask-net only when
-// labels are wanted); warps 0..3, which own TMEM lanes 0..127, take sigma, rgb and the argmax over the Kp logit columns and
-// store sigma / rgb / label.  Nothing [n, K]-shaped leaves the SM.  With live_ids the tile loop stops at the device-side live
-// count (*n_live_in), the way desc.n_valid bounds the training forward.
+// The fused extraction: the per-sample field CTA with a voxel front and an argmax epilogue.  The gather warps turn row s into a
+// voxel (live_ids[s], or voxel s when every voxel is evaluated) and its point, and gather both tables and the SH row of the one
+// view direction; the chain warps run the full mlp_chain (mask-net only when labels are wanted); warps 0..3, which own TMEM
+// lanes 0..127, take sigma, rgb and the argmax over the Kp logit columns and store sigma / rgb / label.  Nothing [n, K]-shaped
+// leaves the SM.  With live_ids the tile loop stops at the device-side live count (*n_live_in), the way desc.n_valid bounds
+// the training forward.
+struct ExtractJob {
+    VolGeom g;
+    const int32_t* live_ids;
+    const int32_t* n_live_in;
+    float vx, vy, vz, sigma_thresh;
+    float* sigma_out;
+    float* rgb_out;
+    int32_t* label_out;
+    int32_t* n_live_out;
+
+    __device__ __forceinline__ uint32_t rows(const inerf_field_desc&) const {   // block 0 also reports the count
+        const uint32_t n = live_ids ? (uint32_t)max(0, __ldg(n_live_in)) : g.n_vox;
+        if (n_live_out && blockIdx.x == 0 && threadIdx.x == 0) *n_live_out = (int32_t)n;
+        return n;
+    }
+    __device__ __forceinline__ void point(uint32_t s, float p[3]) const {
+        uint32_t v[3];
+        vol_voxel(g, live_ids ? (uint32_t)__ldg(live_ids + s) : s, v);
+        vol_point(g, v, p);
+    }
+    __device__ __forceinline__ void sh_row(uint32_t, uint8_t* smem, uint32_t a_ci, uint32_t row) const { sh16_to_smem(vx, vy, vz, smem, a_ci, row); }
+    template <typename Sync>
+    __device__ __forceinline__ void tile(const inerf_field_desc& desc, uint8_t* smem, const ChainBufs& bufs, uint32_t tmem_base, uint64_t* mma_bar,
+                                         uint32_t& phase, uint64_t* release, Sync&& chain_sync, uint32_t row0, uint32_t n, uint32_t tid) const {
+        const uint32_t K = desc.K, Kp = weight_layout(K).Kp;
+        const uint32_t warp = tid >> 5;
+        const bool with_masks = label_out != nullptr;
+        const float sigma = mlp_chain(smem, bufs, tmem_base, mma_bar, phase, K, desc.density_scale, with_masks, tid, release, chain_sync, [](float) {});
+        if (warp < 4) {   // thread tid owns tile row tid
+            float rgb[3];
+            epilogue_rgb(tmem_base, rgb, tid);
+            uint32_t arg = 0;
+            if (with_masks) {
+                // argmax over the fp16-rounded logits inerf_field_forward stores; the lowest index wins a tie
+                float best = 0.f;
+                for (uint32_t c = 0; c < Kp / 16; c++) {
+                    uint32_t v[16];
+                    umma::tmem_ld16(tmem_base + D_d + ((warp * 32u) << 16) + c * 16, v);
+                    umma::tmem_ld_wait();
+#pragma unroll
+                    for (uint32_t i = 0; i < 16; i++) {
+                        const uint32_t k = c * 16 + i;
+                        const float l = __half2float(__float2half_rn(__uint_as_float(v[i])));
+                        if (k < K && (k == 0 || l > best)) { best = l; arg = k; }
+                    }
+                }
+            }
+            const uint32_t s = row0 + tid;
+            if (s < n) {
+                const uint32_t o = live_ids ? (uint32_t)__ldg(live_ids + s) : s;
+                if (sigma_out) sigma_out[o] = sigma;
+                if (rgb_out) { rgb_out[(size_t)o * 3] = rgb[0]; rgb_out[(size_t)o * 3 + 1] = rgb[1]; rgb_out[(size_t)o * 3 + 2] = rgb[2]; }
+                if (label_out) label_out[o] = sigma >= sigma_thresh ? (int32_t)arg + 1 : 0;
+            }
+        }
+    }
+};
+
 __global__ void __launch_bounds__(kWsThreads, 1) k_extract_volume(inerf_field_desc desc, VolGeom g, const int32_t* __restrict__ live_ids,
                                                                   const int32_t* __restrict__ n_live_in, float vx, float vy, float vz,
                                                                   float sigma_thresh, float* __restrict__ sigma_out, float* __restrict__ rgb_out,
                                                                   int32_t* __restrict__ label_out, int32_t* __restrict__ n_live_out) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const uint32_t K = desc.K, Kp = weight_layout(K).Kp;
-    WsCtrl* ctl = reinterpret_cast<WsCtrl*>(smem + WsSmem::ctrl(K));
-    const uint32_t tid = threadIdx.x;
-    load_weights(smem, WsSmem::W, desc.weights, K);
-    init_levels(ctl->lg, desc.offsets, desc.L, desc.S, desc.H, tid);
-    if (tid == 0) {
-        for (uint32_t i = 0; i < kWsStages; i++) { umma::mbar_init(&ctl->a_full[i], kWsGatherT / 32); umma::mbar_init(&ctl->a_empty[i], 1); }
-        umma::mbar_init(&ctl->mma_bar, 1);
-        umma::mbar_fence_init();
-    }
-    if (tid < 32) umma::tmem_alloc<kTmemCols>(&ctl->tmem_slot);
-    umma::fence_async_smem();
-    umma::fence_before_sync();
-    __syncthreads();
-    umma::fence_after_sync();
-    const uint32_t tmem_base = ctl->tmem_slot;
-    const uint32_t n = live_ids ? (uint32_t)max(0, __ldg(n_live_in)) : g.n_vox;
-    const uint32_t num_tiles = (n + kTile - 1) / kTile;
-    const bool with_masks = label_out != nullptr;
-    if (n_live_out && blockIdx.x == 0 && tid == 0) *n_live_out = (int32_t)n;
-
-    if (tid < kWsChainT) {
-        umma::reg_alloc<96>();
-        const uint32_t warp = tid >> 5;
-        uint32_t phase = 0, it = 0;
-        auto chain_sync = [] { umma::named_sync<1, kWsChainT>(); };
-        for (uint32_t tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, it++) {
-            const uint32_t sa = it % kWsStages;
-            umma::mbar_wait(&ctl->a_full[sa], (it / kWsStages) & 1u);
-            const uint32_t a_es = WsSmem::A + sa * kStageBytes;
-            const ChainBufs bufs{a_es, a_es + kBytesEs, a_es + kBytesEs + kBytesCi, WsSmem::W};
-            const float sigma = mlp_chain(smem, bufs, tmem_base, &ctl->mma_bar, phase, K, desc.density_scale, with_masks, tid, &ctl->a_empty[sa],
-                                          chain_sync, [](float) {});
-            if (warp < 4) {   // thread tid owns tile row tid
-                float rgb[3];
-                epilogue_rgb(tmem_base, rgb, tid);
-                uint32_t arg = 0;
-                if (with_masks) {
-                    // argmax over the fp16-rounded logits inerf_field_forward stores; the lowest index wins a tie
-                    float best = 0.f;
-                    for (uint32_t c = 0; c < Kp / 16; c++) {
-                        uint32_t v[16];
-                        umma::tmem_ld16(tmem_base + D_d + ((warp * 32u) << 16) + c * 16, v);
-                        umma::tmem_ld_wait();
-#pragma unroll
-                        for (uint32_t i = 0; i < 16; i++) {
-                            const uint32_t k = c * 16 + i;
-                            const float l = __half2float(__float2half_rn(__uint_as_float(v[i])));
-                            if (k < K && (k == 0 || l > best)) { best = l; arg = k; }
-                        }
-                    }
-                }
-                const uint32_t s = tile * kTile + tid;
-                if (s < n) {
-                    const uint32_t o = live_ids ? (uint32_t)__ldg(live_ids + s) : s;
-                    if (sigma_out) sigma_out[o] = sigma;
-                    if (rgb_out) { rgb_out[(size_t)o * 3] = rgb[0]; rgb_out[(size_t)o * 3 + 1] = rgb[1]; rgb_out[(size_t)o * 3 + 2] = rgb[2]; }
-                    if (label_out) label_out[o] = sigma >= sigma_thresh ? (int32_t)arg + 1 : 0;
-                }
-            }
-            umma::fence_before_sync();
-            chain_sync();   // TMEM and the chain's hidden tiles are reused by the next tile
-        }
-    } else {
-        umma::reg_dealloc<64>();
-        const uint32_t gt = tid - kWsChainT, row = gt & (kTile - 1), quarter = gt >> 7;
-        const float inv2b = __fdiv_rn(1.0f, __fmul_rn(2.0f, desc.bound));
-        const uint2* table = reinterpret_cast<const uint2*>(desc.table_packed);
-        uint32_t it = 0;
-        for (uint32_t tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, it++) {
-            const uint32_t sa = it % kWsStages;
-            if (it >= kWsStages) umma::mbar_wait(&ctl->a_empty[sa], ((it / kWsStages) - 1u) & 1u);
-            const uint32_t s = tile * kTile + row;
-            if (s < n) {   // rows past the end keep stale operands: their outputs are never stored
-                uint32_t v[3];
-                vol_voxel(g, live_ids ? (uint32_t)__ldg(live_ids + s) : s, v);
-                const uint32_t a_es = WsSmem::A + sa * kStageBytes, a_ci = a_es + kBytesEs, a_mi = a_ci + kBytesCi;
-                float p[3], x01[3];
-                vol_point(g, v, p);
-                bool oob = false;
-#pragma unroll
-                for (int d = 0; d < 3; d++) {
-                    x01[d] = __fmul_rn(__fadd_rn(p[d], desc.bound), inv2b);  // grid.py:149
-                    oob |= (x01[d] < 0.f || x01[d] > 1.f);
-                }
-                if (quarter == 0) sh16_to_smem(vx, vy, vz, smem, a_ci, row);
-                encode4(x01, oob, quarter * 4, ctl->lg, table, smem, a_es, a_mi, row);
-            }
-            umma::fence_async_smem();
-            __syncwarp();
-            if ((gt & 31u) == 0) umma::mbar_arrive(&ctl->a_full[sa]);   // one arrival per gather warp
-        }
-    }
-    umma::fence_before_sync();
-    __syncthreads();
-    if (tid < 32) umma::tmem_dealloc<kTmemCols>(tmem_base);
+    ws_field_cta(desc, ExtractJob{g, live_ids, n_live_in, vx, vy, vz, sigma_thresh, sigma_out, rgb_out, label_out, n_live_out});
 }
 
 // fp32 / fp16 embeddings of both encoders -> interleaved fp16 (sigma.c0, sigma.c1, mask.c0, mask.c1), one pass
@@ -452,24 +412,6 @@ __global__ void k_pack_tables(const T* __restrict__ es, const T* __restrict__ em
         }
         out[i] = make_uint2(h2_bits(a), h2_bits(b));
     }
-}
-
-inline uint16_t f2h_bits(float f) {
-    const __half h = __float2half_rn(f);
-    uint16_t b;
-    memcpy(&b, &h, 2);
-    return b;
-}
-
-// W is [n_out, n_in] row-major fp32 -> B-operand tile [Npad x Kpad] with zero padding
-void pack_layer(uint8_t* dst, const float* W, uint32_t n_out, uint32_t n_in, uint32_t Npad, uint32_t Kpad) {
-    const uint32_t sbo = sbo_of(Kpad);
-    for (uint32_t n = 0; n < Npad; n++)
-        for (uint32_t k = 0; k < Kpad; k++) {
-            const float v = (n < n_out && k < n_in) ? W[(size_t)n * n_in + k] : 0.f;
-            const uint16_t b = f2h_bits(v);
-            memcpy(dst + umma::tile_off(n, k, kLBO, sbo), &b, 2);
-        }
 }
 
 int validate_desc(const inerf_field_desc* d) {
@@ -529,26 +471,6 @@ extern "C" int inerf_field_pack_tables(const void* emb_sigma, const void* emb_ma
 
 extern "C" size_t inerf_field_weights_bytes(uint32_t K) { return (K == 0 || K > 64) ? 0 : field::weight_layout(K).total; }
 
-extern "C" int inerf_field_pack_weights(const float* sigma0, const float* sigma1, const float* color0, const float* color1,
-                                        const float* color2, const float* mask0, const float* mask1, const float* mask2, uint32_t K,
-                                        void* packed_host) {
-    if (K == 0 || K > 64) return INERF_ERR_SIZE;
-    INERF_REQUIRE(sigma0); INERF_REQUIRE(sigma1); INERF_REQUIRE(color0); INERF_REQUIRE(color1); INERF_REQUIRE(color2);
-    INERF_REQUIRE(mask0); INERF_REQUIRE(mask1); INERF_REQUIRE(mask2); INERF_REQUIRE(packed_host);
-    const field::WeightLayout wl = field::weight_layout(K);
-    uint8_t* p = static_cast<uint8_t*>(packed_host);
-    memset(p, 0, wl.total);
-    pack_layer(p + wl.s0, sigma0, 64, 32, 64, 32);
-    pack_layer(p + wl.s1, sigma1, 16, 64, 16, 64);
-    pack_layer(p + wl.c0, color0, 64, 31, 64, 32);
-    pack_layer(p + wl.c1, color1, 64, 64, 64, 64);
-    pack_layer(p + wl.c2, color2, 3, 64, 16, 64);
-    pack_layer(p + wl.m0, mask0, 64, 47, 64, 48);
-    pack_layer(p + wl.m1, mask1, 64, 64, 64, 64);
-    pack_layer(p + wl.m2, mask2, K, 64, wl.Kp, 64);
-    return INERF_OK;
-}
-
 static int field_forward_impl(const inerf_field_desc* desc, const float* xyzs, const float* dirs, uint32_t B, float* sigmas, float* rgbs,
                               float* masks, void* x0_save, void* stream, void* xs_save = nullptr) {
     if (int e = validate_desc(desc)) return e;
@@ -556,16 +478,8 @@ static int field_forward_impl(const inerf_field_desc* desc, const float* xyzs, c
     INERF_REQUIRE(xyzs); INERF_REQUIRE(dirs); INERF_REQUIRE(sigmas); INERF_REQUIRE(rgbs);
     if (x0_save && (((uintptr_t)x0_save & 15u) || masks == nullptr)) return INERF_ERR_ALIGN;
     if (xs_save && ((uintptr_t)xs_save & 15u)) return INERF_ERR_ALIGN;
-    const uint32_t num_tiles = (B + field::kTile - 1) / field::kTile;
-    // per-device attribute, cheap to set: no process-global "already done" flag
-    cudaError_t e = cudaFuncSetAttribute(k_field_forward_ws, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-    if (e != cudaSuccess) return (int)e;
-    const uint32_t sms = (uint32_t)device_sm_count();
-    const uint32_t grid_ws = num_tiles < sms ? num_tiles : sms;
-    k_field_forward_ws<<<grid_ws, kWsThreads, WsSmem::bytes(desc->K), (cudaStream_t)stream>>>(*desc, xyzs, dirs, B, sigmas, rgbs, masks,
-                                                                                             (uint4*)x0_save, (uint4*)xs_save);
-    INERF_LAUNCH_CHECK();
-    return INERF_OK;
+    return launch_persistent(k_field_forward_ws, B, kWsThreads, WsSmem::bytes(desc->K), (cudaStream_t)stream, *desc, xyzs, dirs, B, sigmas, rgbs,
+                             masks, (uint4*)x0_save, (uint4*)xs_save);
 }
 
 extern "C" int inerf_occupancy_density(const inerf_field_desc* desc, uint32_t C, uint32_t G, const int32_t* cells, uint32_t per_cascade,
@@ -574,13 +488,8 @@ extern "C" int inerf_occupancy_density(const inerf_field_desc* desc, uint32_t C,
     occ::OccPoints pts;
     if (int e = occ::make_points(&pts, C, G, desc->bound, cells, per_cascade, noise, seed)) return e;
     INERF_REQUIRE(tmp_grid);
-    const uint32_t n = C * per_cascade, num_tiles = (n + field::kTile - 1) / field::kTile;
-    cudaError_t ce = cudaFuncSetAttribute(k_occupancy_density, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-    if (ce != cudaSuccess) return (int)ce;
-    const uint32_t sms = (uint32_t)device_sm_count();
-    k_occupancy_density<<<num_tiles < sms ? num_tiles : sms, kWsThreads, WsSmem::bytes(desc->K), (cudaStream_t)stream>>>(*desc, pts, n, tmp_grid);
-    INERF_LAUNCH_CHECK();
-    return INERF_OK;
+    const uint32_t n = C * per_cascade;
+    return launch_persistent(k_occupancy_density, n, kWsThreads, WsSmem::bytes(desc->K), (cudaStream_t)stream, *desc, pts, n, tmp_grid);
 }
 
 extern "C" int inerf_field_forward(const inerf_field_desc* desc, const float* xyzs, const float* dirs, uint32_t B, float* sigmas,
@@ -644,11 +553,6 @@ extern "C" int inerf_extract_volume(const inerf_field_desc* desc, const float* b
         live_ids = scratch;
         n_live_in = counts + nblk;
     }
-    cudaError_t ce = cudaFuncSetAttribute(k_extract_volume, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-    if (ce != cudaSuccess) return (int)ce;
-    const uint32_t num_tiles = (g.n_vox + field::kTile - 1) / field::kTile, sms = (uint32_t)device_sm_count();
-    k_extract_volume<<<num_tiles < sms ? num_tiles : sms, kWsThreads, WsSmem::bytes(desc->K), st>>>(
-        *desc, g, live_ids, n_live_in, vd[0], vd[1], vd[2], sigma_thresh, sigma, rgb, label, n_live);
-    INERF_LAUNCH_CHECK();
-    return INERF_OK;
+    return launch_persistent(k_extract_volume, g.n_vox, kWsThreads, WsSmem::bytes(desc->K), st, *desc, g, live_ids, n_live_in, vd[0], vd[1], vd[2],
+                             sigma_thresh, sigma, rgb, label, n_live);
 }

@@ -228,25 +228,45 @@ __device__ __forceinline__ void scatter_role(const inerf_field_desc& desc, const
     }
 }
 
-// Two roles per CTA: the CHAIN warps (threads 0..255) run the tcgen05 recompute / dX / dW chain of tile i + 1 while the SCATTER
-// warps (threads 256..511) push tile i's feature gradients into the table gradient.  The scatter is bound by the rate at
-// which an SM retires RED lanes (~1 per clock); run back to back with the chain (the first version of this kernel) it left
-// the tensor pipe and the LSU idle in turns.  dF travels through a double-buffered fp32 tile in shared memory.
-__global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_mask(inerf_field_desc desc, BwdParams p) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const uint32_t K = desc.K, tid = threadIdx.x;
-    LevelGeom* lg = reinterpret_cast<LevelGeom*>(smem + BSmem::MISC);
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem + BSmem::MISC + 16 * sizeof(LevelGeom));
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + BSmem::MISC + 16 * sizeof(LevelGeom) + 8);
-    uint64_t* df_full = reinterpret_cast<uint64_t*>(smem + BSmem::MISC + 16 * sizeof(LevelGeom) + 16);    // [2]
-    uint64_t* df_empty = df_full + 2;                                                                       // [2]
+// ---- CTA of the two backward kernels --------------------------------------------------------------------------------------------
+// Shared memory (Sm = BSmem or RSm): operand tiles [0, Sm::W), the packed weight blob (kWeightBytes) at Sm::W, the dF tiles at
+// Sm::DF and at Sm::MISC: LevelGeom[16] | MMA mbarrier | TMEM slot | df_full[2] | df_empty[2].  512 TMEM columns.
+struct BwdCta {
+    LevelGeom* lg;
+    uint64_t* bar;        // MMA completion (chain role)
+    uint64_t* df_full;    // [2] dF tile written by the chain role
+    uint64_t* df_empty;   // [2] dF tile read by the scatter role
+    uint32_t tmem;
+    uint32_t phase;       // of `bar`
 
-    // zero the operand tiles once (TG2's right half and dY's padding columns stay zero for the whole launch)
-    for (uint32_t i = tid; i < BSmem::W / 16; i += kBwdThreads) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0u, 0u, 0u, 0u);
+    __device__ __forceinline__ void wait_mma() {
+        __syncwarp();
+        umma::mbar_wait(bar, phase);
+        phase ^= 1u;
+        umma::fence_after_sync();
+    }
+    // generic-proxy tile writes -> visible to the next MMAs (barrier over the chain role only)
+    __device__ __forceinline__ void publish() const {
+        umma::fence_async_smem();
+        umma::fence_before_sync();
+        umma::named_sync<1, kBwdChainT>();
+    }
+};
+
+template <typename Sm, uint32_t kWeightBytes>
+__device__ __forceinline__ BwdCta bwd_cta_setup(uint8_t* smem, const inerf_field_desc& desc, const void* weights, uint32_t tid) {
+    LevelGeom* lg = reinterpret_cast<LevelGeom*>(smem + Sm::MISC);
+    uint64_t* bar = reinterpret_cast<uint64_t*>(smem + Sm::MISC + 16 * sizeof(LevelGeom));
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + Sm::MISC + 16 * sizeof(LevelGeom) + 8);
+    uint64_t* df_full = reinterpret_cast<uint64_t*>(smem + Sm::MISC + 16 * sizeof(LevelGeom) + 16);
+    uint64_t* df_empty = df_full + 2;
+
+    // zero the operand tiles once: padding columns that no stage writes stay zero for the whole launch
+    for (uint32_t i = tid; i < Sm::W / 16; i += kBwdThreads) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0u, 0u, 0u, 0u);
     {
-        const uint4* wsrc = reinterpret_cast<const uint4*>(p.weights);
-        uint4* wdst = reinterpret_cast<uint4*>(smem + BSmem::W);
-        for (uint32_t i = tid; i < BwdWeights::total / 16; i += kBwdThreads) wdst[i] = __ldg(wsrc + i);
+        const uint4* wsrc = reinterpret_cast<const uint4*>(weights);
+        uint4* wdst = reinterpret_cast<uint4*>(smem + Sm::W);
+        for (uint32_t i = tid; i < kWeightBytes / 16; i += kBwdThreads) wdst[i] = __ldg(wsrc + i);
     }
     init_levels(lg, desc.offsets, desc.L, desc.S, desc.H, tid);
     if (tid == 0) {
@@ -259,7 +279,25 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_mask(inerf_fi
     umma::fence_before_sync();
     __syncthreads();
     umma::fence_after_sync();
-    const uint32_t tmem = *tmem_slot;
+    return BwdCta{lg, bar, df_full, df_empty, *tmem_slot, 0u};
+}
+
+__device__ __forceinline__ void bwd_cta_teardown(uint32_t tmem, uint32_t tid) {
+    umma::fence_before_sync();
+    __syncthreads();
+    if (tid < 32) umma::tmem_dealloc<kBwdTmemCols>(tmem);
+}
+
+// Two roles per CTA: the CHAIN warps (threads 0..255) run the tcgen05 recompute / dX / dW chain of tile i + 1 while the SCATTER
+// warps (threads 256..511) push tile i's feature gradients into the table gradient.  The scatter is bound by the rate at
+// which an SM retires RED lanes (~1 per clock); run back to back with the chain (the first version of this kernel) it left
+// the tensor pipe and the LSU idle in turns.  dF travels through a double-buffered fp32 tile in shared memory.
+__global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_mask(inerf_field_desc desc, BwdParams p) {
+    extern __shared__ __align__(1024) uint8_t smem[];
+    const uint32_t K = desc.K, tid = threadIdx.x;
+    // TG2's right half and dY's padding columns stay zero
+    BwdCta cta = bwd_cta_setup<BSmem, BwdWeights::total>(smem, desc, p.weights, tid);
+    const uint32_t tmem = cta.tmem;
     const uint32_t sbase = umma::smem_u32(smem);
 
     const bool chain_role = tid < kBwdChainT;
@@ -267,23 +305,10 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_mask(inerf_fi
     const uint32_t warp = rt >> 5, lane = rt & 31;
     const uint32_t row = rt & (kTile - 1), half = rt >> 7;
     const uint32_t lane_base = ((warp & 3u) * 32u) << 16;
-    const float inv2b = __fdiv_rn(1.0f, __fmul_rn(2.0f, desc.bound));
     const uint32_t B_eff = desc.n_valid ? min(p.B, (uint32_t)max(0, __ldg(desc.n_valid))) : p.B;   // rows past *n_valid are padding
     const uint32_t num_tiles = (B_eff + kTile - 1) / kTile;
-    uint32_t phase = 0, tiles_done = 0;
+    uint32_t tiles_done = 0;
     const bool issue_warp = tid < 32;   // one elected lane of warp 0 issues the MMAs (uniform branch for the compiler)
-
-    auto wait_mma = [&] {
-        __syncwarp();
-        umma::mbar_wait(bar, phase);
-        phase ^= 1u;
-        umma::fence_after_sync();
-    };
-    auto publish = [&] {   // generic-proxy tile writes -> visible to the next MMAs (barrier over the chain role only)
-        umma::fence_async_smem();
-        umma::fence_before_sync();
-        umma::named_sync<1, kBwdChainT>();
-    };
 
     if (chain_role) {
     umma::reg_alloc<kBwdRegsChain>();
@@ -343,57 +368,57 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_mask(inerf_fi
                 *reinterpret_cast<uint4*>(smem + BSmem::TG + umma::tile_off(row, k0, kLBO, kSbo128)) = make_uint4(q[0], q[1], q[2], q[3]);
             }
         }
-        publish();
+        cta.publish();
         // ---- S1: H1 pre-activation and dY W2 -----------------------------------------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, BSmem::TX, kSbo48, BSmem::W + BwdWeights::w0, kSbo48, 48, 64, tmem + T_a);
             issue_gemm2(sbase, BSmem::TG, kSbo128, BSmem::W + BwdWeights::w2t, kSbo64, 64, 64, tmem + T_b);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
         prefetch(tile + gridDim.x);   // next tile's inputs: in flight during the four MMA stages of this one
-        wait_mma();
+        cta.wait_mma();
         const uint32_t mask1 = epi_relu32(tmem + T_a + lane_base + half * 32, smem, BSmem::TH, row, 64 + half * 32);   // H1 -> TH[:, 64:128]
-        publish();
+        cta.publish();
         // ---- S2: H2 pre-activation; dH2 = (dY W2) . [H2 > 0] ---------------------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, BSmem::TH + 8 * kLBO, kSbo128, BSmem::W + BwdWeights::w1, kSbo64, 64, 64, tmem + T_a);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
-        wait_mma();
+        cta.wait_mma();
         const uint32_t mask2 = epi_relu32(tmem + T_a + lane_base + half * 32, smem, BSmem::TH, row, half * 32);        // H2 -> TH[:, 0:64]
         epi_masked32(tmem + T_b + lane_base + half * 32, mask2, smem, BSmem::TG, row, 64 + half * 32);                 // dH2 -> TG[:, 64:128]
-        publish();
+        cta.publish();
         // ---- S3: dH1 = (dH2 W1) . [H1 > 0] --------------------------------------------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, BSmem::TG + 8 * kLBO, kSbo128, BSmem::W + BwdWeights::w1t, kSbo64, 64, 64, tmem + T_b);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
-        wait_mma();
+        cta.wait_mma();
         epi_masked32(tmem + T_b + lane_base + half * 32, mask1, smem, BSmem::TG2, row, half * 32);                     // dH1 -> TG2[:, 0:64]
-        publish();
+        cta.publish();
         // ---- S4: dF = dH1 W0[:, :32]; weight gradients accumulate across tiles ------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, BSmem::TG2, kSbo128, BSmem::W + BwdWeights::w0t, kSbo64, 64, 32, tmem + T_x);
             issue_gemm_tn(sbase, BSmem::TG, kSbo128, BSmem::TH, kSbo128, 128, tmem + T_w1, tiles_done > 0);
             issue_gemm_tn(sbase, BSmem::TG2, kSbo128, BSmem::TX, kSbo48, 48, tmem + T_w0, tiles_done > 0);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
-        wait_mma();
+        cta.wait_mma();
         // ---- hand dF (32 feature gradients / sample, fp32, [column][row] so that neither side has bank conflicts) to the scatter warps
         {
             const uint32_t db = tiles_done & 1u;
-            if (tiles_done >= 2) umma::mbar_wait(&df_empty[db], ((tiles_done >> 1) - 1u) & 1u);
+            if (tiles_done >= 2) umma::mbar_wait(&cta.df_empty[db], ((tiles_done >> 1) - 1u) & 1u);
             uint32_t v[16];
             umma::tmem_ld16(tmem + T_x + lane_base + half * 16, v);
             umma::tmem_ld_wait();
             float* dst = reinterpret_cast<float*>(smem + BSmem::DF) + db * (kTile * 32) + (half * 16) * kTile + row;
 #pragma unroll
             for (int i = 0; i < 16; i++) dst[i * kTile] = __uint_as_float(v[i]);
-            umma::mbar_arrive(&df_full[db]);
+            umma::mbar_arrive(&cta.df_full[db]);
         }
         umma::fence_before_sync();
         umma::named_sync<1, kBwdChainT>();   // TMEM accumulators T_a/T_b/T_x and the operand tiles are reused by the next tile
@@ -434,12 +459,9 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_mask(inerf_fi
     }
     } else {
     umma::reg_dealloc<kBwdRegsScatter>();
-    scatter_role(desc, p.xyzs, p.grad_table, lg, smem + BSmem::DF, df_full, df_empty, num_tiles, B_eff, rt);
+    scatter_role(desc, p.xyzs, p.grad_table, cta.lg, smem + BSmem::DF, cta.df_full, cta.df_empty, num_tiles, B_eff, rt);
     }
-
-    umma::fence_before_sync();
-    __syncthreads();
-    if (tid < 32) umma::tmem_dealloc<kBwdTmemCols>(tmem);
+    bwd_cta_teardown(tmem, tid);
 }
 
 // =================================================================================================================================
@@ -501,31 +523,9 @@ struct RgbBwdParams {
 __global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_rgb(inerf_field_desc desc, RgbBwdParams p) {
     extern __shared__ __align__(1024) uint8_t smem[];
     const uint32_t tid = threadIdx.x;
-    LevelGeom* lg = reinterpret_cast<LevelGeom*>(smem + RSm::MISC);
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem + RSm::MISC + 16 * sizeof(LevelGeom));
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + RSm::MISC + 16 * sizeof(LevelGeom) + 8);
-    uint64_t* df_full = reinterpret_cast<uint64_t*>(smem + RSm::MISC + 16 * sizeof(LevelGeom) + 16);    // [2]
-    uint64_t* df_empty = df_full + 2;                                                                     // [2]
-
-    // zero the operand tiles once: the padding columns of GB (and dP's columns 3..15) stay zero for the whole launch
-    for (uint32_t i = tid; i < RSm::W / 16; i += kBwdThreads) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0u, 0u, 0u, 0u);
-    {
-        const uint4* wsrc = reinterpret_cast<const uint4*>(p.weights);
-        uint4* wdst = reinterpret_cast<uint4*>(smem + RSm::W);
-        for (uint32_t i = tid; i < RgbBwdWeights::total / 16; i += kBwdThreads) wdst[i] = __ldg(wsrc + i);
-    }
-    init_levels(lg, desc.offsets, desc.L, desc.S, desc.H, tid);
-    if (tid == 0) {
-        umma::mbar_init(bar, 1);
-        for (int i = 0; i < 2; i++) { umma::mbar_init(&df_full[i], kBwdChainT); umma::mbar_init(&df_empty[i], kBwdScatterT); }
-        umma::mbar_fence_init();
-    }
-    if (tid < 32) umma::tmem_alloc<kBwdTmemCols>(tmem_slot);
-    umma::fence_async_smem();
-    umma::fence_before_sync();
-    __syncthreads();
-    umma::fence_after_sync();
-    const uint32_t tmem = *tmem_slot;
+    // the padding columns of GB (and dP's columns 3..15) stay zero
+    BwdCta cta = bwd_cta_setup<RSm, RgbBwdWeights::total>(smem, desc, p.weights, tid);
+    const uint32_t tmem = cta.tmem;
     const uint32_t sbase = umma::smem_u32(smem);
 
     const bool chain_role = tid < kBwdChainT;
@@ -535,21 +535,9 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_rgb(inerf_fie
     const uint32_t lane_base = ((warp & 3u) * 32u) << 16;
     const uint32_t B_eff = desc.n_valid ? min(p.B, (uint32_t)max(0, __ldg(desc.n_valid))) : p.B;
     const uint32_t num_tiles = (B_eff + kTile - 1) / kTile;
-    uint32_t phase = 0, tiles_done = 0;
+    uint32_t tiles_done = 0;
     const bool issue_warp = tid < 32;   // one elected lane of warp 0 issues the MMAs (uniform branch for the compiler)
     constexpr uint32_t Wb = RSm::W;
-
-    auto wait_mma = [&] {
-        __syncwarp();
-        umma::mbar_wait(bar, phase);
-        phase ^= 1u;
-        umma::fence_after_sync();
-    };
-    auto publish = [&] {
-        umma::fence_async_smem();
-        umma::fence_before_sync();
-        umma::named_sync<1, kBwdChainT>();
-    };
 
     if (chain_role) {
     umma::reg_alloc<kBwdRegsChain>();
@@ -598,46 +586,46 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_rgb(inerf_fie
             const float e = fminf(fmaxf(pf[1], 3.0590232e-07f), 3269017.4f);
             dh0_bits = (uint32_t)__half_as_ushort(__float2half_rn(__fmul_rn(pf[0], e)));
         }
-        publish();
+        cta.publish();
         // ---- S1: Hs, Hc1 pre-activations; dP Wc2 ---------------------------------------------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, RSm::HB, kSbo160, Wb + RgbBwdWeights::ws0, kSbo32, 32, 64, tmem + R_a);
             issue_gemm2(sbase, RSm::HA + 8 * kLBO, kSbo96, Wb + RgbBwdWeights::wc0, kSbo32, 32, 64, tmem + R_b);
             issue_gemm2(sbase, RSm::GB + 8 * kLBO, kSbo128, Wb + RgbBwdWeights::wc2t, kSbo16, 16, 64, tmem + R_c);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
         prefetch(tile + gridDim.x);
-        wait_mma();
+        cta.wait_mma();
         const uint32_t mask_s = epi_relu_to(tmem + R_a + lane_base + half * 32, smem, RSm::HB, kSbo160, row, 96 + half * 32);    // Hs  -> HB[:, 96:160]
         const uint32_t mask_c1 = epi_relu_to(tmem + R_b + lane_base + half * 32, smem, RSm::HA, kSbo96, row, half * 32);        // Hc1 -> HA[:, 0:64]
-        publish();
+        cta.publish();
         // ---- S2: Hc2 pre-activation; dHc2 = (dP Wc2) . [Hc2 > 0] --------------------------------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, RSm::HA, kSbo96, Wb + RgbBwdWeights::wc1, kSbo64, 64, 64, tmem + R_a);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
-        wait_mma();
+        cta.wait_mma();
         const uint32_t mask_c2 = epi_relu_to(tmem + R_a + lane_base + half * 32, smem, RSm::HB, kSbo160, row, 32 + half * 32);   // Hc2 -> HB[:, 32:96]
         epi_masked32(tmem + R_c + lane_base + half * 32, mask_c2, smem, RSm::GA, row, half * 32);                               // dHc2 -> GA[:, 0:64]
-        publish();
+        cta.publish();
         // ---- S3: dHc1 = (dHc2 Wc1) . [Hc1 > 0] ----------------------------------------------------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, RSm::GA, kSbo128, Wb + RgbBwdWeights::wc1t, kSbo64, 64, 64, tmem + R_b);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
-        wait_mma();
+        cta.wait_mma();
         epi_masked32(tmem + R_b + lane_base + half * 32, mask_c1, smem, RSm::GA, row, 64 + half * 32);                          // dHc1 -> GA[:, 64:128]
-        publish();
+        cta.publish();
         // ---- S4: dCi = dHc1 Wc0; the density head's output gradient dO = [dh0 | dgeo15] ----------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, RSm::GA + 8 * kLBO, kSbo128, Wb + RgbBwdWeights::wc0t, kSbo64, 64, 32, tmem + R_x);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
-        wait_mma();
+        cta.wait_mma();
         if (half == 1) {   // columns 16..31 of dCi: geo15 (column 31 is the zero padding of Ci)
             uint32_t v[16];
             umma::tmem_ld16(tmem + R_x + lane_base + 16, v);
@@ -649,35 +637,35 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_rgb(inerf_fie
             *reinterpret_cast<uint4*>(smem + RSm::GB + umma::tile_off(row, 96, kLBO, kSbo128)) = make_uint4(q[0], q[1], q[2], q[3]);
             *reinterpret_cast<uint4*>(smem + RSm::GB + umma::tile_off(row, 104, kLBO, kSbo128)) = make_uint4(q[4], q[5], q[6], q[7]);
         }
-        publish();
+        cta.publish();
         // ---- S5: dHs = (dO Ws1) . [Hs > 0] ---------------------------------------------------------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, RSm::GB + 12 * kLBO, kSbo128, Wb + RgbBwdWeights::ws1t, kSbo16, 16, 64, tmem + R_a);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
-        wait_mma();
+        cta.wait_mma();
         epi_masked32(tmem + R_a + lane_base + half * 32, mask_s, smem, RSm::GB, row, half * 32);                                // dHs -> GB[:, 0:64]
-        publish();
+        cta.publish();
         // ---- S6: dE = dHs Ws0; weight gradients accumulate across tiles ----------------------------------------------------------
         if (issue_warp && umma::elect_one()) {
             umma::fence_after_sync();
             issue_gemm2(sbase, RSm::GB, kSbo128, Wb + RgbBwdWeights::ws0t, kSbo64, 64, 32, tmem + R_x);
             issue_gemm_tn(sbase, RSm::GA, kSbo128, RSm::HA, kSbo96, 96, tmem + R_w1, tiles_done > 0);
             issue_gemm_tn(sbase, RSm::GB, kSbo128, RSm::HB, kSbo160, 160, tmem + R_w2, tiles_done > 0);
-            umma::commit(bar);
+            umma::commit(cta.bar);
         }
-        wait_mma();
+        cta.wait_mma();
         {
             const uint32_t db = tiles_done & 1u;
-            if (tiles_done >= 2) umma::mbar_wait(&df_empty[db], ((tiles_done >> 1) - 1u) & 1u);
+            if (tiles_done >= 2) umma::mbar_wait(&cta.df_empty[db], ((tiles_done >> 1) - 1u) & 1u);
             uint32_t v[16];
             umma::tmem_ld16(tmem + R_x + lane_base + half * 16, v);
             umma::tmem_ld_wait();
             float* dst = reinterpret_cast<float*>(smem + RSm::DF) + db * (kTile * 32) + (half * 16) * kTile + row;
 #pragma unroll
             for (int i = 0; i < 16; i++) dst[i * kTile] = __uint_as_float(v[i]);
-            umma::mbar_arrive(&df_full[db]);
+            umma::mbar_arrive(&cta.df_full[db]);
         }
         umma::fence_before_sync();
         umma::named_sync<1, kBwdChainT>();
@@ -708,30 +696,15 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_field_backward_rgb(inerf_fie
     }
     } else {
     umma::reg_dealloc<kBwdRegsScatter>();
-    scatter_role(desc, p.xyzs, p.grad_table, lg, smem + RSm::DF, df_full, df_empty, num_tiles, B_eff, rt);
+    scatter_role(desc, p.xyzs, p.grad_table, cta.lg, smem + RSm::DF, cta.df_full, cta.df_empty, num_tiles, B_eff, rt);
     }
-
-    umma::fence_before_sync();
-    __syncthreads();
-    if (tid < 32) umma::tmem_dealloc<kBwdTmemCols>(tmem);
+    bwd_cta_teardown(tmem, tid);
 }
 
-inline uint16_t f2h(float f) {
-    const __half h = __float2half_rn(f);
-    uint16_t b;
-    memcpy(&b, &h, 2);
-    return b;
-}
-// element (n, k) of a [Npad x Kpad] K-major B-operand tile
-inline void put(uint8_t* dst, uint32_t n, uint32_t k, uint32_t Kpad, float v) {
-    const uint16_t b = f2h(v);
-    memcpy(dst + umma::tile_off(n, k, kLBO, sbo_of(Kpad)), &b, 2);
-}
-
-}  // namespace
-
-namespace {
-// ---- on-device weight packing (no host round trip: the trainable weights change every optimizer step) ----------
+// ---- weight packing: fp32 nn.Linear matrices -> the fp16 operand blobs of the field kernels ---------------------------------
+// Each blob is written down once, as a list of PackJobs (one per operand tile).  The host packers (CPU pointers) and
+// k_pack_weights (DEVICE pointers, no host round trip: the trainable weights change every optimizer step) apply the same
+// element rule, pack_value.
 struct PackJob {
     const float* W;        // fp32 [n_out, n_in] row-major (nn.Linear layout)
     uint32_t n_out, n_in;  // logical shape of W
@@ -743,7 +716,19 @@ struct PackJob {
 struct PackJobs {
     PackJob j[13];
     uint32_t n;
+    void add(const float* W, uint32_t n_out, uint32_t n_in, uint32_t Npad, uint32_t Kpad, uint32_t dst, uint32_t tr, uint32_t n_lim) {
+        j[n++] = PackJob{W, n_out, n_in, Npad, Kpad, dst, tr, n_lim};
+    }
 };
+
+// element (n, k) of job J's tile; zero outside W
+__host__ __device__ __forceinline__ float pack_value(const PackJob& J, uint32_t n, uint32_t k) {
+    float v = 0.f;
+    if (!J.transpose) { if (n < J.n_out && k < J.n_in) v = J.W[(size_t)n * J.n_in + k]; }
+    else if (k < J.n_out && n < J.n_in && n < J.n_lim) v = J.W[(size_t)k * J.n_in + n];
+    return v;
+}
+
 __global__ void k_pack_weights(PackJobs jobs, uint8_t* fwd, uint8_t* bwd, uint32_t n_fwd) {
     for (uint32_t ji = blockIdx.y; ji < jobs.n; ji += gridDim.y) {
         const PackJob J = jobs.j[ji];
@@ -751,14 +736,59 @@ __global__ void k_pack_weights(PackJobs jobs, uint8_t* fwd, uint8_t* bwd, uint32
         const uint32_t total = J.Npad * J.Kpad;
         for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
             const uint32_t n = i / J.Kpad, k = i % J.Kpad;
-            float v = 0.f;
-            if (!J.transpose) { if (n < J.n_out && k < J.n_in) v = J.W[(size_t)n * J.n_in + k]; }
-            else if (k < J.n_out && n < J.n_in && n < J.n_lim) v = J.W[(size_t)k * J.n_in + n];
-            *reinterpret_cast<__half*>(out + umma::tile_off(n, k, kLBO, sbo_of(J.Kpad))) = __float2half_rn(v);
+            *reinterpret_cast<__half*>(out + umma::tile_off(n, k, kLBO, sbo_of(J.Kpad))) = __float2half_rn(pack_value(J, n, k));
         }
     }
 }
+
+// every element of every tile: the jobs of a blob cover it, so no byte keeps what was there before
+void pack_on_host(const PackJobs& jobs, uint8_t* blob) {
+    for (uint32_t ji = 0; ji < jobs.n; ji++) {
+        const PackJob& J = jobs.j[ji];
+        for (uint32_t n = 0; n < J.Npad; n++)
+            for (uint32_t k = 0; k < J.Kpad; k++) {
+                const __half h = __float2half_rn(pack_value(J, n, k));
+                memcpy(blob + J.dst + umma::tile_off(n, k, kLBO, sbo_of(J.Kpad)), &h, 2);
+            }
+    }
+}
+
+// the forward blob (field::weight_layout): sigma-net, colour-net, mask-net
+void add_forward_layers(PackJobs& jobs, const float* sigma0, const float* sigma1, const float* color0, const float* color1, const float* color2,
+                        const float* mask0, const float* mask1, const float* mask2, uint32_t K) {
+    const WeightLayout wl = weight_layout(K);
+    jobs.add(sigma0, 64, 32, 64, 32, wl.s0, 0, 64);
+    jobs.add(sigma1, 16, 64, 16, 64, wl.s1, 0, 16);
+    jobs.add(color0, 64, 31, 64, 32, wl.c0, 0, 64);
+    jobs.add(color1, 64, 64, 64, 64, wl.c1, 0, 64);
+    jobs.add(color2, 3, 64, 16, 64, wl.c2, 0, 16);
+    jobs.add(mask0, 64, 47, 64, 48, wl.m0, 0, 64);
+    jobs.add(mask1, 64, 64, 64, 64, wl.m1, 0, 64);
+    jobs.add(mask2, K, 64, wl.Kp, 64, wl.m2, 0, wl.Kp);
+}
+
+// the mask-head backward blob (BwdWeights)
+void add_mask_bwd_layers(PackJobs& jobs, const float* mask0, const float* mask1, const float* mask2, uint32_t K) {
+    jobs.add(mask0, 64, 47, 64, 48, BwdWeights::w0, 0, 64);
+    jobs.add(mask1, 64, 64, 64, 64, BwdWeights::w1, 0, 64);
+    jobs.add(mask2, K, 64, 64, 64, BwdWeights::w2t, 1, 64);
+    jobs.add(mask1, 64, 64, 64, 64, BwdWeights::w1t, 1, 64);
+    jobs.add(mask0, 64, 47, 32, 64, BwdWeights::w0t, 1, 32);
+}
+
 }  // namespace
+
+extern "C" int inerf_field_pack_weights(const float* sigma0, const float* sigma1, const float* color0, const float* color1,
+                                        const float* color2, const float* mask0, const float* mask1, const float* mask2, uint32_t K,
+                                        void* packed_host) {
+    if (K == 0 || K > 64) return INERF_ERR_SIZE;
+    INERF_REQUIRE(sigma0); INERF_REQUIRE(sigma1); INERF_REQUIRE(color0); INERF_REQUIRE(color1); INERF_REQUIRE(color2);
+    INERF_REQUIRE(mask0); INERF_REQUIRE(mask1); INERF_REQUIRE(mask2); INERF_REQUIRE(packed_host);
+    PackJobs jobs{};
+    add_forward_layers(jobs, sigma0, sigma1, color0, color1, color2, mask0, mask1, mask2, K);
+    pack_on_host(jobs, static_cast<uint8_t*>(packed_host));
+    return INERF_OK;
+}
 
 // Device-side equivalent of inerf_field_pack_weights (+ inerf_field_pack_weights_bwd when packed_bwd != NULL):
 // all pointers are DEVICE pointers, one launch, no synchronisation.
@@ -768,30 +798,11 @@ extern "C" int inerf_field_pack_weights_device(const float* sigma0, const float*
     if (K == 0 || K > 64) return INERF_ERR_SIZE;
     INERF_REQUIRE(sigma0); INERF_REQUIRE(sigma1); INERF_REQUIRE(color0); INERF_REQUIRE(color1); INERF_REQUIRE(color2);
     INERF_REQUIRE(mask0); INERF_REQUIRE(mask1); INERF_REQUIRE(mask2); INERF_REQUIRE(packed_fwd);
-    const WeightLayout wl = weight_layout(K);
     PackJobs jobs{};
-    uint32_t n = 0;
-    auto add = [&](const float* W, uint32_t n_out, uint32_t n_in, uint32_t Npad, uint32_t Kpad, uint32_t dst, uint32_t tr, uint32_t n_lim) {
-        jobs.j[n++] = PackJob{W, n_out, n_in, Npad, Kpad, dst, tr, n_lim};
-    };
-    add(sigma0, 64, 32, 64, 32, wl.s0, 0, 64);
-    add(sigma1, 16, 64, 16, 64, wl.s1, 0, 16);
-    add(color0, 64, 31, 64, 32, wl.c0, 0, 64);
-    add(color1, 64, 64, 64, 64, wl.c1, 0, 64);
-    add(color2, 3, 64, 16, 64, wl.c2, 0, 16);
-    add(mask0, 64, 47, 64, 48, wl.m0, 0, 64);
-    add(mask1, 64, 64, 64, 64, wl.m1, 0, 64);
-    add(mask2, K, 64, wl.Kp, 64, wl.m2, 0, wl.Kp);
-    const uint32_t n_fwd = n;
-    if (packed_bwd) {
-        add(mask0, 64, 47, 64, 48, BwdWeights::w0, 0, 64);
-        add(mask1, 64, 64, 64, 64, BwdWeights::w1, 0, 64);
-        add(mask2, K, 64, 64, 64, BwdWeights::w2t, 1, 64);
-        add(mask1, 64, 64, 64, 64, BwdWeights::w1t, 1, 64);
-        add(mask0, 64, 47, 32, 64, BwdWeights::w0t, 1, 32);
-    }
-    jobs.n = n;
-    k_pack_weights<<<dim3(4, n), 256, 0, (cudaStream_t)stream>>>(jobs, (uint8_t*)packed_fwd, (uint8_t*)packed_bwd, n_fwd);
+    add_forward_layers(jobs, sigma0, sigma1, color0, color1, color2, mask0, mask1, mask2, K);
+    const uint32_t n_fwd = jobs.n;
+    if (packed_bwd) add_mask_bwd_layers(jobs, mask0, mask1, mask2, K);
+    k_pack_weights<<<dim3(4, jobs.n), 256, 0, (cudaStream_t)stream>>>(jobs, (uint8_t*)packed_fwd, (uint8_t*)packed_bwd, n_fwd);
     INERF_LAUNCH_CHECK();
     return INERF_OK;
 }
@@ -801,20 +812,9 @@ extern "C" size_t inerf_field_bwd_weights_bytes(void) { return BwdWeights::total
 extern "C" int inerf_field_pack_weights_bwd(const float* mask0, const float* mask1, const float* mask2, uint32_t K, void* packed_host) {
     if (K == 0 || K > 64) return INERF_ERR_SIZE;
     INERF_REQUIRE(mask0); INERF_REQUIRE(mask1); INERF_REQUIRE(mask2); INERF_REQUIRE(packed_host);
-    uint8_t* p = static_cast<uint8_t*>(packed_host);
-    memset(p, 0, BwdWeights::total);
-    for (uint32_t o = 0; o < 64; o++)
-        for (uint32_t j = 0; j < 47; j++) {
-            put(p + BwdWeights::w0, o, j, 48, mask0[o * 47 + j]);
-            if (j < 32) put(p + BwdWeights::w0t, j, o, 64, mask0[o * 47 + j]);
-        }
-    for (uint32_t o = 0; o < 64; o++)
-        for (uint32_t j = 0; j < 64; j++) {
-            put(p + BwdWeights::w1, o, j, 64, mask1[o * 64 + j]);
-            put(p + BwdWeights::w1t, j, o, 64, mask1[o * 64 + j]);
-        }
-    for (uint32_t o = 0; o < K; o++)
-        for (uint32_t j = 0; j < 64; j++) put(p + BwdWeights::w2t, j, o, 64, mask2[o * 64 + j]);
+    PackJobs jobs{};
+    add_mask_bwd_layers(jobs, mask0, mask1, mask2, K);
+    pack_on_host(jobs, static_cast<uint8_t*>(packed_host));
     return INERF_OK;
 }
 
@@ -826,16 +826,8 @@ extern "C" int inerf_field_backward_mask(const inerf_field_desc* desc, const voi
     INERF_REQUIRE(weights_bwd); INERF_REQUIRE(xyzs); INERF_REQUIRE(x0); INERF_REQUIRE(grad_logits);
     INERF_REQUIRE(grad_table); INERF_REQUIRE(grad_w0); INERF_REQUIRE(grad_w1); INERF_REQUIRE(grad_w2);
     if (((uintptr_t)weights_bwd & 15u) || ((uintptr_t)x0 & 15u) || ((uintptr_t)grad_table & 7u)) return INERF_ERR_ALIGN;
-    // per-device attribute, cheap to set: no process-global "already done" flag
-    cudaError_t e = cudaFuncSetAttribute(k_field_backward_mask, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BSmem::bytes);
-    if (e != cudaSuccess) return (int)e;
-    BwdParams p{xyzs, (const uint4*)x0, grad_logits, B, (float2*)grad_table, grad_w0, grad_w1, grad_w2, weights_bwd};
-    const uint32_t num_tiles = (B + kTile - 1) / kTile;
-    const uint32_t sms = (uint32_t)device_sm_count();
-    const uint32_t grid = num_tiles < sms ? num_tiles : sms;
-    k_field_backward_mask<<<grid, kBwdThreads, BSmem::bytes, (cudaStream_t)stream>>>(*desc, p);
-    INERF_LAUNCH_CHECK();
-    return INERF_OK;
+    const BwdParams p{xyzs, (const uint4*)x0, grad_logits, B, (float2*)grad_table, grad_w0, grad_w1, grad_w2, weights_bwd};
+    return launch_persistent(k_field_backward_mask, B, kBwdThreads, BSmem::bytes, (cudaStream_t)stream, *desc, p);
 }
 
 // ---- stage-1 (RGB-sigma) backward ------------------------------------------------------------------------------------------
@@ -848,20 +840,15 @@ extern "C" int inerf_field_pack_weights_rgb_bwd_device(const float* sigma0, cons
     INERF_REQUIRE(packed_bwd);
     if ((uintptr_t)packed_bwd & 15u) return INERF_ERR_ALIGN;
     PackJobs jobs{};
-    uint32_t n = 0;
-    auto add = [&](const float* W, uint32_t n_out, uint32_t n_in, uint32_t Npad, uint32_t Kpad, uint32_t dst, uint32_t tr, uint32_t n_lim) {
-        jobs.j[n++] = PackJob{W, n_out, n_in, Npad, Kpad, dst, tr, n_lim};
-    };
-    add(sigma0, 64, 32, 64, 32, RgbBwdWeights::ws0, 0, 64);
-    add(color0, 64, 31, 64, 32, RgbBwdWeights::wc0, 0, 64);
-    add(color1, 64, 64, 64, 64, RgbBwdWeights::wc1, 0, 64);
-    add(color2, 3, 64, 64, 16, RgbBwdWeights::wc2t, 1, 64);
-    add(color1, 64, 64, 64, 64, RgbBwdWeights::wc1t, 1, 64);
-    add(color0, 64, 31, 32, 64, RgbBwdWeights::wc0t, 1, 32);
-    add(sigma1, 16, 64, 64, 16, RgbBwdWeights::ws1t, 1, 64);
-    add(sigma0, 64, 32, 32, 64, RgbBwdWeights::ws0t, 1, 32);
-    jobs.n = n;
-    k_pack_weights<<<dim3(4, n), 256, 0, (cudaStream_t)stream>>>(jobs, nullptr, (uint8_t*)packed_bwd, 0);
+    jobs.add(sigma0, 64, 32, 64, 32, RgbBwdWeights::ws0, 0, 64);
+    jobs.add(color0, 64, 31, 64, 32, RgbBwdWeights::wc0, 0, 64);
+    jobs.add(color1, 64, 64, 64, 64, RgbBwdWeights::wc1, 0, 64);
+    jobs.add(color2, 3, 64, 64, 16, RgbBwdWeights::wc2t, 1, 64);
+    jobs.add(color1, 64, 64, 64, 64, RgbBwdWeights::wc1t, 1, 64);
+    jobs.add(color0, 64, 31, 32, 64, RgbBwdWeights::wc0t, 1, 32);
+    jobs.add(sigma1, 16, 64, 64, 16, RgbBwdWeights::ws1t, 1, 64);
+    jobs.add(sigma0, 64, 32, 32, 64, RgbBwdWeights::ws0t, 1, 32);
+    k_pack_weights<<<dim3(4, jobs.n), 256, 0, (cudaStream_t)stream>>>(jobs, nullptr, (uint8_t*)packed_bwd, 0);
     INERF_LAUNCH_CHECK();
     return INERF_OK;
 }
@@ -876,13 +863,7 @@ extern "C" int inerf_field_backward_rgb(const inerf_field_desc* desc, const void
     INERF_REQUIRE(grad_sigmas); INERF_REQUIRE(grad_rgbs); INERF_REQUIRE(grad_table);
     INERF_REQUIRE(grad_ws0); INERF_REQUIRE(grad_ws1); INERF_REQUIRE(grad_wc0); INERF_REQUIRE(grad_wc1); INERF_REQUIRE(grad_wc2);
     if (((uintptr_t)weights_bwd & 15u) || ((uintptr_t)xs & 15u) || ((uintptr_t)grad_table & 15u)) return INERF_ERR_ALIGN;
-    cudaError_t e = cudaFuncSetAttribute(k_field_backward_rgb, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RSm::bytes);
-    if (e != cudaSuccess) return (int)e;
-    RgbBwdParams p{xyzs, (const uint4*)xs, sigmas, rgbs, grad_sigmas, grad_rgbs, B, (float2*)grad_table,
-                   grad_ws0, grad_ws1, grad_wc0, grad_wc1, grad_wc2, weights_bwd};
-    const uint32_t num_tiles = (B + kTile - 1) / kTile;
-    const uint32_t sms = (uint32_t)device_sm_count();
-    k_field_backward_rgb<<<num_tiles < sms ? num_tiles : sms, kBwdThreads, RSm::bytes, (cudaStream_t)stream>>>(*desc, p);
-    INERF_LAUNCH_CHECK();
-    return INERF_OK;
+    const RgbBwdParams p{xyzs, (const uint4*)xs, sigmas, rgbs, grad_sigmas, grad_rgbs, B, (float2*)grad_table,
+                         grad_ws0, grad_ws1, grad_wc0, grad_wc1, grad_wc2, weights_bwd};
+    return launch_persistent(k_field_backward_rgb, B, kBwdThreads, RSm::bytes, (cudaStream_t)stream, *desc, p);
 }

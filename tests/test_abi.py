@@ -68,6 +68,34 @@ def test_pack_weights_layout_roundtrip(L):
     assert base == n
 
 
+@pytest.mark.parametrize("K", [5, 16, 64])
+def test_pack_weights_bwd_layout(L, K):
+    """Host-side packing of the mask-head backward blob, every byte: five [Npad x Kpad] K-major tiles, element (n, k) at
+    the same offset as in the forward round trip.  W0, W1 as they are; W2, W1, W0[:, :32] transposed, (n, k) = W[k][n],
+    with zeros where the output index k >= K (W2) and in every padding row or column."""
+    import numpy as np
+    rng = np.random.RandomState(1)
+    m0, m1, m2 = (np.ascontiguousarray(rng.randn(*s).astype(np.float32)) for s in [(64, 47), (64, 64), (K, 64)])
+    n = L.inerf_field_bwd_weights_bytes()
+    blob = np.full(n, 0xA5, np.uint8)   # not zero: the packer must write every byte
+    assert L.inerf_field_pack_weights_bwd(m0.ctypes.data, m1.ctypes.data, m2.ctypes.data, K, blob.ctypes.data) == 0
+    h = blob.view(np.float16)
+    base = 0
+    for i, (src, Np, Kp) in enumerate([(m0, 64, 48), (m1, 64, 64), (m2.T, 64, 64), (m1.T, 64, 64), (m0.T, 32, 64)]):
+        n_, k_ = np.meshgrid(np.arange(Np), np.arange(Kp), indexing="ij")
+        got = h[base // 2 + ((n_ % 8) * 16 + (n_ // 8) * ((Kp // 8) * 128) + (k_ // 8) * 128 + (k_ % 8) * 2) // 2]
+        want = np.zeros((Np, Kp), np.float16)
+        r, c = min(Np, src.shape[0]), min(Kp, src.shape[1])
+        want[:r, :c] = src[:r, :c]
+        assert np.array_equal(got.view(np.uint16), want.view(np.uint16))
+        if i == 2:
+            assert not np.any(got[:, K:])   # transposed W2: output index o >= K is zero
+        base += Np * Kp * 2
+    assert base == n
+    assert L.inerf_field_pack_weights_bwd(m0.ctypes.data, m1.ctypes.data, m2.ctypes.data, 0, blob.ctypes.data) == -2
+    assert L.inerf_field_pack_weights_bwd(None, m1.ctypes.data, m2.ctypes.data, K, blob.ctypes.data) == -1
+
+
 def test_product_path_has_no_cpu_fallback():
     import torch
     from instance_nerf_b200 import raymarching

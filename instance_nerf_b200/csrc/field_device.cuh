@@ -110,8 +110,28 @@ __device__ __forceinline__ void init_levels(LevelGeom* lg, const int32_t* __rest
     }
 }
 
+// Class of the 4 consecutive levels [l0, l0 + 4) a gather thread encodes: all dense, all hashed with a power-of-two size
+// (the hash-grid preset: levels 0..3 dense, 4..15 hashed), or mixed.  The levels of a gather warp are fixed, so the branch on
+// the class is warp-uniform and the dense and hashed quarters run straight-line code without a mode branch per level.
+constexpr uint32_t kLevelsMixed = 0, kLevelsDense = 1, kLevelsHashed = 2;
+__device__ __forceinline__ uint32_t level_class4(const LevelGeom* lg, uint32_t l0) {
+    const uint32_t m0 = lg[l0].mode, m1 = lg[l0 + 1].mode, m2 = lg[l0 + 2].mode, m3 = lg[l0 + 3].mode;
+    if ((m0 | m1 | m2 | m3) == 0u) return kLevelsDense;
+    if (m0 == 1u && m1 == 1u && m2 == 1u && m3 == 1u) return kLevelsHashed;
+    return kLevelsMixed;
+}
+
+// (a ^ b) & m as one three-input LOP3 (left to itself the compiler forms x ^ y ^ z per corner and masks it separately)
+__device__ __forceinline__ uint32_t xor_and(uint32_t a, uint32_t b, uint32_t m) {
+    uint32_t r;
+    asm("lop3.b32 %0, %1, %2, %3, 0x28;" : "=r"(r) : "r"(a), "r"(b), "r"(m));
+    return r;
+}
+
 // Corner indices (relative to the level's first entry) and trilinear weights of one point at one level.
 // w fp32 = (wx * wy) * wz in the reference's order (gridencoder.cu:161-185 / :283-301).
+// kMode: the level's mode when the caller knows it (0 dense, 1 hashed with a power-of-two size); -1 reads g.mode.
+template <int kMode = -1>
 __device__ __forceinline__ void level_corners(const float x01[3], const LevelGeom& g, uint32_t idx[8], float w[8]) {
     float fr[3];
     uint32_t pg[3];
@@ -126,7 +146,8 @@ __device__ __forceinline__ void level_corners(const float x01[3], const LevelGeo
     const float wy[2] = {__fsub_rn(1.0f, fr[1]), fr[1]};
     const float wz[2] = {__fsub_rn(1.0f, fr[2]), fr[2]};
     // one warp-uniform branch per level (dense levels never wrap, hashed levels have power-of-two sizes)
-    if (g.mode == 0) {
+    const uint32_t mode = kMode < 0 ? g.mode : (uint32_t)kMode;
+    if (mode == 0) {
         const uint32_t y0 = pg[1] * g.r1, y1 = y0 + g.r1, z0 = pg[2] * g.r1sq, z1 = z0 + g.r1sq;
         const uint32_t b00 = pg[0] + y0 + z0, b10 = pg[0] + y1 + z0, b01 = pg[0] + y0 + z1, b11 = pg[0] + y1 + z1;
         idx[0] = b00; idx[1] = b00 + 1u; idx[2] = b10; idx[3] = b10 + 1u;
@@ -135,9 +156,9 @@ __device__ __forceinline__ void level_corners(const float x01[3], const LevelGeo
         const uint32_t x0 = pg[0], x1 = pg[0] + 1u;
         const uint32_t y0 = pg[1] * 2654435761u, y1 = y0 + 2654435761u, z0 = pg[2] * 805459861u, z1 = z0 + 805459861u;
         const uint32_t h00 = y0 ^ z0, h10 = y1 ^ z0, h01 = y0 ^ z1, h11 = y1 ^ z1;
-        idx[0] = (x0 ^ h00) & g.mask; idx[1] = (x1 ^ h00) & g.mask; idx[2] = (x0 ^ h10) & g.mask; idx[3] = (x1 ^ h10) & g.mask;
-        idx[4] = (x0 ^ h01) & g.mask; idx[5] = (x1 ^ h01) & g.mask; idx[6] = (x0 ^ h11) & g.mask; idx[7] = (x1 ^ h11) & g.mask;
-        if (g.mode == 2) {   // hashed level whose size is not a power of two (never produced by grid.py's level table; kept exact)
+        idx[0] = xor_and(x0, h00, g.mask); idx[1] = xor_and(x1, h00, g.mask); idx[2] = xor_and(x0, h10, g.mask); idx[3] = xor_and(x1, h10, g.mask);
+        idx[4] = xor_and(x0, h01, g.mask); idx[5] = xor_and(x1, h01, g.mask); idx[6] = xor_and(x0, h11, g.mask); idx[7] = xor_and(x1, h11, g.mask);
+        if (kMode < 0 && mode == 2) {   // hashed level whose size is not a power of two (never produced by grid.py's level table; kept exact)
             idx[0] = (x0 ^ h00) % g.size; idx[1] = (x1 ^ h00) % g.size; idx[2] = (x0 ^ h10) % g.size; idx[3] = (x1 ^ h10) % g.size;
             idx[4] = (x0 ^ h01) % g.size; idx[5] = (x1 ^ h01) % g.size; idx[6] = (x0 ^ h11) % g.size; idx[7] = (x1 ^ h11) % g.size;
         }
@@ -151,19 +172,30 @@ __device__ __forceinline__ void level_corners(const float x01[3], const LevelGeo
 // Per corner: product rounded to fp16; fp16 accumulation.
 // __hadd2 (one rounding of the exact sum) equals the reference's half(float(acc) + float(p)): fp32 carries
 // 24 >= 2*11+2 bits, so the double rounding is innocuous.
-__device__ __forceinline__ void encode_level(const float x01[3], const LevelGeom g, const uint2* __restrict__ table, uint32_t& out_s,
+template <int kMode = -1>
+__device__ __forceinline__ void encode_level(const float x01[3], const LevelGeom& g, const uint2* __restrict__ table, uint32_t& out_s,
                                              uint32_t& out_m) {
     uint32_t idx[8];
     float w[8];
-    level_corners(x01, g, idx, w);
-    const uint2* base = table + g.offset;
+    level_corners<kMode>(x01, g, idx, w);
+    // Addresses: the entry index offset + idx is formed in 32 bits -- it is below offsets[L], an int32 -- so a corner costs one
+    // 32-bit add and one widening shift-add onto the table base, not a 64-bit add of level base and index.  The x-neighbour of a
+    // dense corner is the next entry (idx[c + 1] = idx[c] + 1 never wraps): the same address + 8 bytes, an immediate offset of
+    // the load.
+    const uint2* ptr[8];
+    const uint32_t mode = kMode < 0 ? g.mode : (uint32_t)kMode;
+#pragma unroll
+    for (uint32_t c = 0; c < 8; c += 2) {
+        ptr[c] = table + (g.offset + idx[c]);
+        ptr[c + 1] = mode == 0 ? ptr[c] + 1 : table + (g.offset + idx[c + 1]);
+    }
     uint2 v[8];
     // One 8-byte gather per corner.  (Tried and rejected on B200: fetching the x-neighbour with one aligned 16-byte gather when
     // it is entry a^1 -- 23 % fewer L1 sectors but LDG.128 scatters cost as many data-pipe wavefronts, +6 % time; DESIGN.md 4.1.)
     // (Also rejected on B200: L1::no_allocate for the finest levels -- 9.5 -> 14.5 ms per c2 frame: the x-neighbour of a corner
     // is fetched by the next instruction of the same thread and hits the line the first one allocated.)
 #pragma unroll
-    for (uint32_t c = 0; c < 8; c++) v[c] = __ldg(base + idx[c]);
+    for (uint32_t c = 0; c < 8; c++) v[c] = __ldg(ptr[c]);
     __half2 as = __float2half2_rn(0.f), am = as;
 #pragma unroll
     for (uint32_t c = 0; c < 8; c++) {
@@ -179,28 +211,35 @@ __device__ __forceinline__ void encode_level(const float x01[3], const LevelGeom
     out_m = h2_bits(am);
 }
 
-// Encode 4 consecutive levels [l0, l0+4) of one point: one 16-byte core-matrix row chunk per table.
+// Encode 4 consecutive levels [l0, l0+4) of one point, the 4 + 4 packed feature pairs returned in registers.
+// (The class is read from shared memory per call: held in a register across the render kernel's tile loop it costs the
+// 64-register gather warps a spill.)
+__device__ __forceinline__ void encode4_regs(const float x01[3], bool oob, uint32_t l0, const LevelGeom* __restrict__ lg,
+                                             const uint2* __restrict__ table, uint32_t (&fs)[4], uint32_t (&fm)[4]) {
+    const uint32_t cls = level_class4(lg, l0);
+    if (cls == kLevelsHashed) {
+#pragma unroll
+        for (uint32_t li = 0; li < 4; li++) encode_level<1>(x01, lg[l0 + li], table, fs[li], fm[li]);
+    } else if (cls == kLevelsDense) {
+#pragma unroll
+        for (uint32_t li = 0; li < 4; li++) encode_level<0>(x01, lg[l0 + li], table, fs[li], fm[li]);
+    } else {
+#pragma unroll
+        for (uint32_t li = 0; li < 4; li++) encode_level(x01, lg[l0 + li], table, fs[li], fm[li]);
+    }
+#pragma unroll
+    for (uint32_t li = 0; li < 4; li++)
+        if (oob) { fs[li] = 0u; fm[li] = 0u; }
+}
+
+// Same, stored as one 16-byte core-matrix row chunk per table of the shared-memory operand stage.
 __device__ __forceinline__ void encode4(const float x01[3], bool oob, uint32_t l0, const LevelGeom* __restrict__ lg,
                                         const uint2* __restrict__ table, uint8_t* smem, uint32_t a_es, uint32_t a_mi, uint32_t row) {
     uint32_t fs[4], fm[4];
-#pragma unroll
-    for (uint32_t li = 0; li < 4; li++) {
-        encode_level(x01, lg[l0 + li], table, fs[li], fm[li]);
-        if (oob) { fs[li] = 0u; fm[li] = 0u; }
-    }
+    encode4_regs(x01, oob, l0, lg, table, fs, fm);
     const uint32_t k0 = l0 * 2;
     *reinterpret_cast<uint4*>(smem + a_es + umma::tile_off(row, k0, kLBO, sbo_of(32))) = make_uint4(fs[0], fs[1], fs[2], fs[3]);
     *reinterpret_cast<uint4*>(smem + a_mi + umma::tile_off(row, k0, kLBO, sbo_of(48))) = make_uint4(fm[0], fm[1], fm[2], fm[3]);
-}
-
-// Same, the 4 + 4 packed feature pairs returned in registers (the render kernel stores them to tensor memory itself)
-__device__ __forceinline__ void encode4_regs(const float x01[3], bool oob, uint32_t l0, const LevelGeom* __restrict__ lg,
-                                             const uint2* __restrict__ table, uint32_t (&fs)[4], uint32_t (&fm)[4]) {
-#pragma unroll
-    for (uint32_t li = 0; li < 4; li++) {
-        encode_level(x01, lg[l0 + li], table, fs[li], fm[li]);
-        if (oob) { fs[li] = 0u; fm[li] = 0u; }
-    }
 }
 
 // SH degree 4 (same polynomials as shencode.cu) rounded to fp16 into A_ci columns 0..15

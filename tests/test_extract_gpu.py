@@ -10,7 +10,7 @@ from test_field_gpu import build_model
 
 pytestmark = pytest.mark.gpu
 
-SUB = (-2.9, -1.45, -2.4, 2.5, 1.3, 2.2)     # a sub-box of the synthetic room (bound 8)
+SUB = (-2.9, -1.45, -2.4, 2.5, 1.3, 2.2)     # a sub-box of the synthetic room (bound 8; scaled by bound / 8 at other bounds)
 SHAPE = (37, 20, 53)                          # non-cubic, no axis a multiple of 4 or 8
 VD = tuple(float(v) for v in (np.array([0.3, -0.5, 0.8]) / np.linalg.norm([0.3, -0.5, 0.8])).astype(np.float32))
 
@@ -49,13 +49,15 @@ def _expected(m, xyzs, thr):
     return s, c, lab
 
 
-@pytest.mark.parametrize("K,density_scale", [(32, 1.0), (16, 25.0), (2, 1.0), (48, 1.0)])
-def test_dense_bit_identical_to_field_forward(cuda, K, density_scale):
-    m, _ = build_model(cuda, K, density_scale=density_scale)
-    xyzs, _ = _points(m, SHAPE, SUB)
+@pytest.mark.parametrize("K,density_scale,bound", [(32, 1.0, 8.0), (16, 25.0, 8.0), (2, 1.0, 8.0), (48, 1.0, 8.0), (16, 25.0, 2.0)],
+                         ids=["32-1.0", "16-25.0", "2-1.0", "48-1.0", "16-25.0-bound2"])
+def test_dense_bit_identical_to_field_forward(cuda, K, density_scale, bound):
+    m, _ = build_model(cuda, K, bound=bound, density_scale=density_scale)
+    sub = tuple(v * bound / 8 for v in SUB)
+    xyzs, _ = _points(m, SHAPE, sub)
     s_ref = m.forward_fused(xyzs, torch.tensor(VD, device=cuda).expand(xyzs.shape[0], 3).contiguous(), want_masks=False)[0]
     thr = float((s_ref * density_scale).median())       # both sides of the label test are populated
-    v = m.extract_volume(SHAPE, bbox=SUB, view_dir=VD, sigma_thresh=thr, skip_empty=False)
+    v = m.extract_volume(SHAPE, bbox=sub, view_dir=VD, sigma_thresh=thr, skip_empty=False)
     s, c, lab = _expected(m, xyzs, thr)
     assert v["sigma"].shape == SHAPE and v["rgb"].shape == (*SHAPE, 3) and v["label"].shape == SHAPE and v["label"].dtype == torch.int32
     assert bits_equal(v["sigma"].view(-1), s)

@@ -23,12 +23,14 @@ def build_model(cuda, K=32, bound=8.0, seed=0, density_scale=1.0):
     return m.to(cuda).eval(), sc
 
 
-@pytest.mark.parametrize("K,B", [(32, 128 * 37 + 5), (16, 1000), (2, 64), (48, 300)])
-def test_field_fused_vs_modular(cuda, K, B):
-    m, _ = build_model(cuda, K)
+# bound 2 (the reference's default): levels 4-7 form a mixed quarter, which the fused kernels encode on their generic path
+@pytest.mark.parametrize("K,B,bound", [(32, 128 * 37 + 5, 8.0), (16, 1000, 8.0), (2, 64, 8.0), (48, 300, 8.0), (32, 128 * 37 + 5, 2.0)],
+                         ids=["32-4741", "16-1000", "2-64", "48-300", "32-4741-bound2"])
+def test_field_fused_vs_modular(cuda, K, B, bound):
+    m, _ = build_model(cuda, K, bound=bound)
     g = torch.Generator().manual_seed(1)
-    x = ((torch.rand(B, 3, generator=g) * 2 - 1) * 7.9).to(cuda)
-    x[:4] = torch.tensor([[8.0, -8.0, 0.0], [0.0, 0.0, 0.0], [8.0, 8.0, 8.0], [-8.0, -8.0, -8.0]], device=cuda)
+    x = ((torch.rand(B, 3, generator=g) * 2 - 1) * 7.9 * bound / 8).to(cuda)
+    x[:4] = torch.tensor([[1.0, -1.0, 0.0], [0.0, 0.0, 0.0], [1.0, 1.0, 1.0], [-1.0, -1.0, -1.0]], device=cuda) * bound
     d = torch.nn.functional.normalize(torch.randn(B, 3, generator=g), dim=-1).to(cuda)
     with torch.no_grad():
         s1, c1, k1 = m.forward_fused(x, d)
@@ -72,11 +74,13 @@ def _render_both(m, o, d, **kw):
     return r1, r0
 
 
-@pytest.mark.parametrize("K,density_scale", [(32, 1.0), (16, 25.0)])
-def test_render_fused_vs_reference_loop(cuda, K, density_scale):
+@pytest.mark.parametrize("K,density_scale,bound", [(32, 1.0, 8.0), (16, 25.0, 8.0), (16, 25.0, 2.0), (16, 25.0, 3.0)],
+                         ids=["32-1.0", "16-25.0", "16-25.0-bound2", "16-25.0-bound3"])
+def test_render_fused_vs_reference_loop(cuda, K, density_scale, bound):
     """Whole-frame inference: the one-launch fused renderer against the reference's alive-ray loop
-    (mask_renderer.py:330-381) run on the op-level kernels.  North-star tolerance: maps within 1e-3."""
-    m, sc = build_model(cuda, K, density_scale=density_scale)
+    (mask_renderer.py:330-381) run on the op-level kernels.  North-star tolerance: maps within 1e-3.  Bound 2 has 2 cascades,
+    bound 3 has 3 with the coarsest one clipped to the box, and both encode levels 4-7 as a mixed quarter."""
+    m, sc = build_model(cuda, K, bound=bound, density_scale=density_scale)
     o, d = make_rays(sc, 96, 128)
     o, d = o.to(cuda), d.to(cuda)
     r1, r0 = _render_both(m, o, d, dt_gamma=1 / 128, max_steps=1024, T_thresh=1e-4)
@@ -157,8 +161,17 @@ def test_update_extra_state_full_sweep_vs_oracle(cuda):
     threshold -> packbits) with injected jitter, against the CPU restatement: a sample of cells per cascade is recomputed
     on the host (query point from the Morton index and the cell's row of the jitter block, fp32 field) and the whole
     grid -> (mean, bitfield) tail is recomputed from the GPU grid with the numpy EMA / packbits restatement (bit-exact)."""
+    _full_sweep_vs_oracle(cuda, 8.0)
+
+
+def test_update_extra_state_full_sweep_vs_oracle_bound2(cuda):
+    """The same at bound 2 (2 cascades), where the sweep kernel encodes levels 4-7 as a mixed quarter."""
+    _full_sweep_vs_oracle(cuda, 2.0)
+
+
+def _full_sweep_vs_oracle(cuda, bound):
     from oracle import field_oracle as fo
-    m, _ = build_model(cuda, 8, density_scale=1.0)
+    m, _ = build_model(cuda, 8, bound=bound, density_scale=1.0)
     m.train()
     m.reset_extra_state()
     G, C = m.grid_size, m.cascade

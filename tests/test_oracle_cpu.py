@@ -138,6 +138,79 @@ def test_grid_encode_and_sh_against_reference_kernels(gk):
     np.testing.assert_allclose(sh.numpy(), gk["sh_out"], rtol=1e-6, atol=1e-7)
 
 
+# Level modes of GridEncoder(desired_resolution=2048 * bound) with the device's level scales: 0 dense, 1 hashed.  At bounds 1-3
+# level 4 is dense and 5-7 hashed, so every fused kernel runs its mixed-quarter (generic per-level) path on levels 4-7.
+LEVEL_CLASSES = {
+    1: ("0000011111111111", ["dense", "mixed", "hashed", "hashed"]),
+    2: ("0000011111111111", ["dense", "mixed", "hashed", "hashed"]),
+    3: ("0000011111111111", ["dense", "mixed", "hashed", "hashed"]),
+    8: ("0000111111111111", ["dense", "hashed", "hashed", "hashed"]),
+}
+
+
+@pytest.mark.parametrize("bound", sorted(LEVEL_CLASSES))
+def test_level_classes_from_recorded_scales(gk, bound):
+    offsets, _ = fo.level_offsets(desired_resolution=2048 * bound)
+    modes, classes = fo.level_modes(offsets, gk[f"enc_scales_b{bound}"])
+    assert ("".join(map(str, modes)), classes) == LEVEL_CLASSES[bound]
+
+
+def test_fma_f32_rounds_once():
+    """pos = fmaf(x01, scale, 0.5): a * b = 2^-25 + 2^-57 (641 * 6700417 = 2^32 + 1) puts the float64 sum exactly on the float32
+    midpoint 0.5 + 2^-25; the exact value lies above it, so one rounding gives 0.5 + 2^-24 where float64-then-float32 gives 0.5."""
+    a, b = np.float32(641 * 2.0 ** -30), np.float32(6700417 * 2.0 ** -27)
+    assert np.float32(float(a) * float(b) + 0.5) == np.float32(0.5)
+    assert fo.fma_f32(np.array([a]), b, 0.5)[0] == np.float32(0.5 + 2.0 ** -24)
+    assert fo.fma_f32(np.array([-a]), b, 0.5)[0] == np.float32(0.5 - 2.0 ** -25)
+    x = np.random.RandomState(0).rand(10000).astype(np.float32)
+    assert np.array_equal(fo.fma_f32(x, np.float32(47.502937), 0.5), (x.astype(np.float64) * float(np.float32(47.502937)) + 0.5).astype(np.float32))
+
+
+def _f16_error_bound(x01, table, offsets, scales):
+    """|fp16 encode - exact| <= 16 half-ulps of the largest partial sum: 8 product roundings + 8 accumulation roundings."""
+    big = np.abs(fo.grid_encode(torch.from_numpy(x01), torch.from_numpy(np.abs(table)), offsets, 2.0, scales=scales).numpy())
+    return 16 * 2.0 ** -11 * np.maximum(big, 2.0 ** -14)
+
+
+def test_grid_encode_half_matches_reference_kernel_fp32(gk):
+    """The fp16 oracle on the reference kernel's bound-2 inputs against the reference's fp32 output: within fp16 error, so its
+    corner indices and weights are the reference's at bound 2 (dense, mixed and hashed quarters)."""
+    offsets, _ = fo.level_offsets(desired_resolution=2048 * 2)
+    T = int(offsets[-1])
+    table = (torch.rand(T, 2, generator=torch.Generator().manual_seed(int(gk["enc_table_seed"][0]))) - 0.5).numpy()
+    x01, scales = gk["enc_x01"], gk["enc_scales_b2"]
+    h = fo.grid_encode_half(x01, table.astype(np.float16), offsets, scales)
+    assert h.dtype == np.float16 and h.shape == gk["enc_out"].shape
+    err = np.abs(h.astype(np.float64) - gk["enc_out"])
+    assert (err <= _f16_error_bound(x01, table, offsets, scales)).all(), float(err.max())
+    assert float(err.mean()) < 1e-4
+    assert not h[2].any()                                                 # out-of-range input -> zeros
+
+
+def test_grid_encode_half_non_power_of_two_hashed_levels(gk):
+    """Hashed levels whose size is not a power of two (mode 2: `% size`) inside the mixed quarter and a hashed one: the fp16
+    oracle against the fp32 one, within fp16 error."""
+    offsets, pls = fo.level_offsets(desired_resolution=2048 * 2)
+    scales = gk["enc_scales_b2"]
+    sizes = np.diff(offsets.astype(np.int64))
+    for l, n in ((6, 3 << 17), (7, 5 << 16), (13, 3 << 17)):
+        sizes[l] = n
+    offs = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int32)
+    modes, classes = fo.level_modes(offs, scales)
+    assert [modes[l] for l in (4, 5, 6, 7, 13)] == [0, 1, 2, 2, 2] and classes == ["dense", "mixed", "hashed", "mixed"]
+    g = torch.Generator().manual_seed(11)
+    table = ((torch.rand(int(offs[-1]), 2, generator=g) - 0.5).numpy()).astype(np.float16)
+    x01 = torch.rand(2000, 3, generator=g).numpy()
+    h = fo.grid_encode_half(x01, table, offs, scales)
+    ref = fo.grid_encode(torch.from_numpy(x01), torch.from_numpy(table.astype(np.float32)), offs, pls, scales=scales).numpy()
+    err = np.abs(h.astype(np.float64) - ref)
+    assert (err <= _f16_error_bound(x01, table.astype(np.float32), offs, scales)).all(), float(err.max())
+    # the `% size` levels really differ from a power-of-two mask of the same size
+    idx, _ = fo.level_corners_np(x01, offs, scales, 6)
+    rel = idx - offs[6]
+    assert (rel < sizes[6]).all() and (rel >= 1 << 18).any()
+
+
 def test_grid_encode_constant_table_and_gradcheck():
     """Analytic checks of SURVEY.md section 8c: constant table -> constant output; fp64 finite differences."""
     offsets, pls = fo.level_offsets(num_levels=4, base_resolution=4, log2_hashmap_size=8, desired_resolution=32)

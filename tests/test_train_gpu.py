@@ -20,13 +20,14 @@ def _rel(a, b):
     return float((a - b).norm() / b.norm().clamp(min=1e-12))
 
 
-@pytest.mark.parametrize("K,B", [(32, 128 * 9 + 17), (16, 128 * 3), (5, 77)])
-def test_fused_backward_matches_autograd(cuda, K, B):
-    m, _ = build_model(cuda, K)
+@pytest.mark.parametrize("K,B,bound", [(32, 128 * 9 + 17, 8.0), (16, 128 * 3, 8.0), (5, 77, 8.0), (32, 128 * 9 + 17, 2.0)],
+                         ids=["32-1169", "16-384", "5-77", "32-1169-bound2"])
+def test_fused_backward_matches_autograd(cuda, K, B, bound):
+    m, _ = build_model(cuda, K, bound=bound)
     m.train()
     _freeze(m)
     g = torch.Generator().manual_seed(3)
-    x = ((torch.rand(B, 3, generator=g) * 2 - 1) * 7.5).to(cuda)
+    x = ((torch.rand(B, 3, generator=g) * 2 - 1) * 7.5 * bound / 8).to(cuda)
     d = torch.nn.functional.normalize(torch.randn(B, 3, generator=g), dim=-1).to(cuda)
     G = torch.randn(B, K, generator=g).to(cuda)
     params = [m.encoder_mask.embeddings, *[l.weight for l in m.mask_net]]
